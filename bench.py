@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference's CPU path (port)
+    python bench.py --dump-outputs DIR ...                          # + the last timed step's obs, rew, done as DIR/*.npy
 
 A "step" is ONE launch of the single-step kernel (MR_Env.step for every env of the rank) on
 synthetic random actions: fp64 storage, sigma = 1 (MR_Env.reset default) drawn by the in-kernel
@@ -34,6 +35,10 @@ METRIC = "env_steps_per_sec"
 UNIT = "env-steps/s"
 BYTES_PER_ENV_STEP = {"f64": 153, "f32": 81}     # SURVEY.md §8(d): algorithmic bytes, single-step path
 PREROLL_S = 0.1     # the timed kernel runs back to back this long (untimed) right before ev0: clocks ramped, caches warm
+# With --dump-outputs the pre-roll is this many launches instead (0.06 s at 2^20 fp64 envs, B200 at 1000 W): the env
+# state carries over from step to step, so the dumped step must have the same number of steps before it in every run.
+DUMP_PREROLL_LAUNCHES = 2048
+DUMP_BUDGET_BYTES = 60 << 20      # array bytes: with the .npy headers a dump stays under 64 MB, even of 10^6 bytes
 
 
 def parse():
@@ -56,7 +61,15 @@ def parse():
     ap.add_argument("--preroll-s", type=float, default=PREROLL_S,
                     help="seconds of the timed kernel run back to back right before the timed region (shrink it for an ncu pass)")
     ap.add_argument("--no-extras", action="store_true", help="skip the fused-rollout / small-batch side numbers")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (obs, rew, done of every env) as DIR/<name>.npy; "
+                         "the pre-roll then has a fixed length, so the same arguments give the same arrays in every run")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 # ---- clocks during the timed region -----------------------------------------------------------
@@ -202,6 +215,20 @@ def run_ours(args):
             return [float(x) for x in t.tolist()]
         return [v]
 
+    def gather_rows(t):
+        """[n, ...] rows of every rank, in env order, as one numpy array on rank 0 (None elsewhere)."""
+        t = t.contiguous()
+        if world == 1:
+            return t.cpu().numpy()
+        sizes = [torch.zeros(1, dtype=torch.int64, device=dev) for _ in range(world)]
+        dist.all_gather(sizes, torch.tensor([t.shape[0]], dtype=torch.int64, device=dev))
+        m = max(int(s) for s in sizes)
+        padded = torch.zeros((m, *t.shape[1:]), dtype=t.dtype, device=dev)
+        padded[:t.shape[0]] = t
+        parts = [torch.empty_like(padded) for _ in range(world)]
+        dist.all_gather(parts, padded)
+        return torch.cat([p[:int(s)] for p, s in zip(parts, sizes)]).cpu().numpy() if rank == 0 else None
+
     strong = args.scaling == "strong"
     n_total = args.envs
     from mr_rl_b200 import shard_range
@@ -233,7 +260,8 @@ def run_ours(args):
         """W warm-up steps, then the SAME kernel back to back for >= preroll_s (still untimed: the clocks ramp and
         settle under load), then — with no synchronisation or idle gap after the last pre-roll launch — ev0, exactly
         `steps` single-step launches, ev1.  use_graph: the K launches are one CUDA-graph replay (captured once; the
-        pre-roll replays the same graph).  Returns (ms of the K steps, wall-clock window, pre-roll launches)."""
+        pre-roll replays the same graph).  Returns (ms of the K steps, wall-clock window from the start of the pre-roll,
+        pre-roll launches, ms of the pre-roll, graph, what the last step returned)."""
         preroll_s = args.preroll_s if preroll_s is None else preroll_s
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -244,14 +272,17 @@ def run_ours(args):
         p1.record()
         torch.cuda.synchronize()
         per = max(p0.elapsed_time(p1) / W, 1e-3)              # ms per launch, rough (cold)
-        n_pre = int(min(20000, max(8, preroll_s * 1e3 / per)))
+        n_pre = DUMP_PREROLL_LAUNCHES if args.dump_outputs else int(min(20000, max(8, preroll_s * 1e3 / per)))
         barrier()
+        t_pre = time.perf_counter()
+        p0.record()
         if g is not None:
-            for _ in range(max(2, n_pre // steps)):
+            n_pre = max(2, n_pre // steps) * steps            # whole replays of the K-step graph
+            for _ in range(n_pre // steps):
                 g.replay()
             t0 = time.perf_counter()
             e0.record()
-            g.replay()
+            out = g.replay()
             e1.record()
         else:
             for k in range(n_pre):
@@ -259,12 +290,12 @@ def run_ours(args):
             t0 = time.perf_counter()
             e0.record()
             for k in range(steps):
-                e.step(a[k % pool])
+                out = e.step(a[k % pool])
             e1.record()
         torch.cuda.synchronize()
         t1 = time.perf_counter()
         barrier()
-        return e0.elapsed_time(e1), (t0, t1), n_pre, g
+        return e0.elapsed_time(e1), (t_pre, t1), n_pre, p0.elapsed_time(e0), g, out
 
     # ---- headline: BASELINE configs[2] as written — `envs` envs sharded over the ranks, single-step path ---------------
     use_graph = args.launch == "graph" or (args.launch == "auto" and n < (1 << 20))
@@ -273,7 +304,9 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_local, (t_wall0, t_wall1), n_pre, graph = timed_steps(env, acts, K, use_graph)
+    ms_local, (t_wall0, t_wall1), n_pre, ms_pre, graph, last = timed_steps(env, acts, K, use_graph)
+    if args.dump_outputs:                                     # the next launch overwrites these buffers: copy them now
+        last = {"obs": gather_rows(last[0]), "rew": gather_rows(last[1]), "done": gather_rows(last[2])}
     per_rank_ms = all_ranks(ms_local / K)
     ms = max_over_ranks(ms_local)
     launches = K + (1 if use_graph else 0)                   # kernels inside the timed region (graph: + the counter kernel)
@@ -293,7 +326,6 @@ def run_ours(args):
     # the timed region lasts a few ms — shorter than nvidia-smi's sampling period — so the same kernel
     # keeps running (untimed) for ~0.4 s while the clock sampler collects its under-load samples
     if rank == 0:
-        t_wall0 -= args.preroll_s
         t_ext = time.perf_counter()
         while time.perf_counter() - t_ext < 0.4:
             if graph is not None:
@@ -305,7 +337,8 @@ def run_ours(args):
         t_wall1 = time.perf_counter()
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     if clocks is not None:
-        clocks["window"] = "0.1 s pre-roll + timed region + 0.4 s of the same kernel back to back (20 ms nvidia-smi period)"
+        clocks["window"] = ("%.3f s pre-roll (%d launches) + timed region + 0.4 s of the same kernel back to back "
+                            "(20 ms nvidia-smi period)" % (ms_pre * 1e-3, n_pre))
     barrier()
     env.check_status()
 
@@ -397,7 +430,7 @@ def run_ours(args):
         def weak():
             ew = make_env(1 << 20, rank * (1 << 20))
             aw = make_actions(1 << 20, 99 + rank)
-            msw, _, _, _ = timed_steps(ew, aw, K, False)
+            msw = timed_steps(ew, aw, K, False)[0]
             msw = max_over_ranks(msw) / K
             extras["weak_scaling_1M_envs_per_gpu"] = {
                 "value": world * (1 << 20) / (msw * 1e-3), "unit": UNIT, "ms_per_step": msw, "envs_total": world << 20,
@@ -406,7 +439,7 @@ def run_ours(args):
         side("weak_scaling_1M_envs_per_gpu", weak)
     if use_graph and not args.no_extras:
         def direct():
-            msd, _, _, _ = timed_steps(env, acts, K, False)
+            msd = timed_steps(env, acts, K, False)[0]
             msd = max_over_ranks(msd) / K
             extras["same_steps_without_cuda_graph"] = {"value": envs_all / (msd * 1e-3), "unit": UNIT, "ms_per_step": msd}
         side("same_steps_without_cuda_graph", direct)
@@ -415,7 +448,7 @@ def run_ours(args):
         # the same single-step kernel with sigma = 0 (MR_simulator.py:18 default noise_var): no RNG work
         def noise_free():
             env0 = make_env(n, base, sigma=0.0)
-            ms0_local, _, _, _ = timed_steps(env0, acts, K, use_graph)
+            ms0_local = timed_steps(env0, acts, K, use_graph)[0]
             ms0 = max_over_ranks(ms0_local) / K
             ach0 = bytes_per_launch / (ms0 * 1e-3) / 1e9
             extras["noise_free_sigma0"] = {"value": envs_all / (ms0 * 1e-3), "unit": UNIT, "ms_per_step": ms0,
@@ -425,7 +458,7 @@ def run_ours(args):
     if not args.no_extras:
         def with_sp():
             env.want_state_prime = True
-            mss, _, _, _ = timed_steps(env, acts, K, False)
+            mss = timed_steps(env, acts, K, False)[0]
             env.want_state_prime = False
             mss = max_over_ranks(mss) / K
             b = (BYTES_PER_ENV_STEP[args.dtype] + 2 * el) * n
@@ -479,9 +512,28 @@ def run_ours(args):
             "clocks": clocks, "repeat_ms_per_step": repeats, "per_rank_ms_per_step": per_rank_ms, "preroll_launches": n_pre,
             "episode_stats_allreduced": stats, **extras,
         }
+        if args.dump_outputs:
+            line["dumped_outputs"] = write_outputs(args.dump_outputs, last)
         print(json.dumps(line), file=_OUT, flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def write_outputs(dirname, arrays):
+    """Write each [n, ...] array as dirname/<name>.npy, float64 kept and anything else as float32.  If the set is larger
+    than DUMP_BUDGET_BYTES, every array keeps the same fixed, seeded sample of rows, whose indices go to env_index.npy.
+    Returns {name: shape}."""
+    import numpy as np
+    arrays = {k: v.astype(v.dtype if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(v[:1].nbytes for v in arrays.values())
+    if n * row_bytes > DUMP_BUDGET_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BUDGET_BYTES // (row_bytes + 8), replace=False))
+        arrays = {"env_index": rows.astype(np.float64), **{k: v[rows] for k, v in arrays.items()}}
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), np.ascontiguousarray(v))
+    return {k: list(v.shape) for k, v in arrays.items()}
 
 
 def _static_traffic(key):

@@ -328,6 +328,54 @@ def gen_recording(n_env=3, K=60, max_steps=12):
     np.savez_compressed(os.path.join(GOLDEN_DIR, "recording.npz"), **out)
 
 
+def sweep_regime(seed):
+    """Inputs of random regime `seed` (tests/test_live_reference_sweep.py): all drawn from default_rng(500 + seed)."""
+    rng = np.random.default_rng(500 + seed)
+    n, T = 6, 25
+    scale = float(rng.choice([20.0, 150.0, 4000.0, 7000.0]))
+    sigma = float(rng.choice([0.0, 0.02, 0.05] if scale < 100 else [0.0, 0.05, 0.5, 1.0]))
+    a0 = float(rng.choice([0.5, 1.0, 1.5, 4.0]))
+    mism = bool(rng.integers(0, 2))
+    init = rng.uniform(-scale, scale, (n, 2))
+    acts = np.stack([rng.uniform(-5, 30, (T, n)), rng.uniform(-7, 7, (T, n))], -1)
+    acts[rng.random((T, n)) < 0.05] = 0.0
+    z = rng.standard_normal((n, 200 * T + 64))
+    return dict(n=n, T=T, sigma=sigma, a0=a0, mism=mism, init=init, acts=acts, z=z)
+
+
+def sweep_reference(r):
+    """Step every env of regime `r` through MR_Env: positions [T, n, 2], done [T, n], draws used [n].  The live
+    reference when its tree is present, otherwise oracle/scipy_env.py — the reference's env restated on scipy's RK45,
+    pinned to the live-reference goldens by tests/test_oracle_golden.py.  Returns the arrays and the source's name."""
+    import contextlib
+    import io
+    from .scipy_env import ScipyEnv
+    live = lr.available()
+    pos, done, cursor = np.zeros((r["T"], r["n"], 2)), np.zeros((r["T"], r["n"]), np.uint8), np.zeros(r["n"], np.int64)
+    for i in range(r["n"]):
+        with contextlib.redirect_stdout(io.StringIO()), lr.patched_noise(r["z"][i]) as ns:
+            env = lr.new_env() if live else ScipyEnv(normal=ns)
+            env.reset(r["init"][i].copy(), noise_var=r["sigma"], a0=r["a0"], is_mismatched=r["mism"])
+            for k in range(r["T"]):
+                _, _, d, _ = env.step(r["acts"][k, i].copy())
+                pos[k, i] = np.array(env.last_pos if live else env.y, dtype=np.float64)
+                done[k, i] = bool(d)
+            cursor[i] = ns.cursor
+    return pos, done, cursor, "MR_RL MR_Env (live)" if live else "oracle/scipy_env.py on scipy RK45"
+
+
+def gen_sweep(seeds=6):
+    """The six random regimes of tests/test_live_reference_sweep.py (scale up to 7000, sigma up to 1, a0 in
+    {0.5, 1, 1.5, 4}, mismatch on or off).  The inputs are regenerated from their seeds; stored are the positions,
+    done flags and final noise cursors, and which implementation produced them."""
+    out = {"versions": versions()}
+    for seed in range(seeds):
+        pos, done, cursor, source = sweep_reference(sweep_regime(seed))
+        out[f"seed{seed}/pos"], out[f"seed{seed}/done"], out[f"seed{seed}/cursor"] = pos, done, cursor
+    out["source"] = np.array(source)
+    np.savez_compressed(os.path.join(GOLDEN_DIR, "sweep.npz"), **out)
+
+
 if __name__ == "__main__":
     os.makedirs(GOLDEN_DIR, exist_ok=True)
     import sys
@@ -343,3 +391,4 @@ if __name__ == "__main__":
     gen_learn_2d()
     gen_ddpg_host()
     gen_recording()
+    gen_sweep()

@@ -1,5 +1,5 @@
-"""MRExperiment wire format (MR_data.py) written from rollout arrays; checked against the live reference's
-own logger when /root/reference is available (build container), structurally otherwise."""
+"""MRExperiment wire format (MR_data.py) written from rollout arrays; checked against what the reference's own logger
+recorded (tests/golden/recording.npz), and against the live logger where the reference tree is present."""
 import contextlib
 import io
 
@@ -36,10 +36,32 @@ def test_experiment_dict_structure_roundtrip(tmp_path):
     assert np.array_equal(back["states"][0], exp["states"][0])
 
 
-@pytest.mark.skipif(not lr.available(), reason="needs the unmodified reference (build container)")
 def test_wire_format_equals_the_reference_logger():
-    """Run the live reference with its MRExperiment logger attached (MR_env.py:94-95,190-198) and compare the
-    dict it would pickle with the one built from the trajectory arrays."""
+    """experiment_dict against what the reference's MRExperiment logger (MR_env.py:94-95,190-198) recorded: always the
+    first episode of every env of the golden recording.npz, from the trajectory of the same inputs through the oracle;
+    where the reference tree is present, also a live run with the logger attached, keys and scalars included."""
+    g = _golden_recording()
+    acts, inits, z, max_steps = g["actions"], g["inits"], g["z"], int(g["max_steps"])
+    K, n_env = acts.shape[:2]
+    E = inits.shape[0]
+    xy, done = np.zeros((K, 2, n_env)), np.zeros((K, n_env), bool)
+    for j in range(n_env):
+        s = mo.SimState(noise=mo.NoiseCursor(z[:, j]))
+        mo.env_reset(s, inits[E - 1, j], 1.0, 1.0, False)
+        for k in range(K):
+            obs, _, done[k, j] = mo.env_step(s, acts[k, j], max_steps=max_steps)[:3]
+            xy[k, :, j] = obs[:2]
+    mine = experiment_dict(inits[E - 1], acts, xy, done=done, until_done=True)
+    assert mine["iterations"] == n_env - 1
+    for j in range(n_env):
+        n = int(g[f"env{j}/steps"][0])
+        assert mine["steps"][j] == n, j
+        for key in ("states", "observations", "actions", "rewards"):
+            ref = g[f"env{j}/{key}"][:n + 1]
+            assert mine[key][j].shape == ref.shape, (key, j)
+            assert np.allclose(mine[key][j], ref, rtol=1e-9, atol=1e-12), (key, j)
+    if not lr.available():
+        return
     acts, z, r = _oracle_run()
     mods = lr.load()
     env = lr.new_env()
