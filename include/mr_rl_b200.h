@@ -17,6 +17,7 @@
  *                       (Learning_module.py:10-24,186-224)
  *   mr_gp_correct_heading <- LearningModule.predict's minimize_scalar(objective, 'Bounded')
  *                       (Learning_module.py:215, utils.py:194-196)
+ *   mr_gp_correct_action_2d <- LearningModule2D.predict's minimize over (alpha, f)  (Learning_module_2d.py:239-268)
  *   mr_actor_forward <- ActorNetwork.predict    (RL/MR_ddpg.py:124-149)
  *   mr_ddpg_update, mr_replay_add, mr_ou_noise_add <- the learner of RL/MR_ddpg.py (:16-78, :163-231, :285-305)
  *   mr_learn_preprocess <- LearningModule.estimateDisturbance / learn up to the fit (Learning_module.py:46-59, :63-120)
@@ -308,6 +309,17 @@ int64_t mr_gp_fit_workspace_bytes(int32_t n_pad);
 int mr_gp_correct_heading_cheb(const double* coef_x, const double* coef_y, int32_t n_coef, const double* vd, int64_t n,
                                double a0, double freq, double drift_x, double drift_y, double* alpha_out, int32_t* nfev_out,
                                void* stream);
+
+/* LearningModule2D.predict's search (Learning_module_2d.py:239-268) for n desired velocities vd[n][2]: the minimiser over
+ * (alpha, f) in the box [lo, hi] of |a0 f (cos alpha, sin alpha) + (muX, muY)(alpha, f) - vd|^2 (= the reference's objective),
+ * both GP means and their gradients evaluated on the device, started at clip((atan2(vd), |vd| / a0)).  x_out[n][2];
+ * iters_out[n] (passes used) and status_out[n] (0 converged, 1 pass cap, 2 non-finite) may be NULL.  The posterior at the
+ * minimiser is a following mr_gp_predict call.  lo, hi, a0 are host values; gpx, gpy must be dim-2 models over the same
+ * training inputs.  The search is a projected Newton / Levenberg-Marquardt method on the box (csrc/mr_gp.cu), not a port
+ * of scipy's L-BFGS-B; where the minimum is unique the two end at the same point to within L-BFGS-B's own tolerance. */
+int mr_gp_correct_action_2d(const mr_gp_model* gpx, const mr_gp_model* gpy, const double* vd, int64_t n, double a0,
+                            const double lo[2], const double hi[2], double* x_out, int32_t* iters_out, uint8_t* status_out,
+                            void* stream);
 
 /* ---- DDPG actor forward (RL/MR_ddpg.py:124-149) --------------------------------------
  * Packed float32 parameters (input-major matrices W[in][out]):

@@ -99,7 +99,7 @@ EXPORTS = ("mr_abi_version", "mr_last_error", "mr_default_params", "mr_fill_time
            "mr_critic_param_count", "mr_replay_add", "mr_ou_noise_add", "mr_ddpg_update", "mr_learn_preprocess",
            "mr_learn_workspace_bytes", "mr_ddpg_workspace_bytes", "mr_replay_sample", "mr_actor_forward_env", "mr_ddpg_gradients", "mr_ddpg_apply", "mr_gp_correct_heading_cheb", "mr_host_pipeline_create", "mr_host_pipeline_destroy", "mr_env_step_host",
            "mr_actor_forward", "mr_set_step_path", "mr_env_reset_ex", "mr_counter_set", "mr_set_actor_path",
-           "mr_host_register", "mr_host_unregister", "mr_philox_normals")
+           "mr_host_register", "mr_host_unregister", "mr_philox_normals", "mr_gp_correct_action_2d")
 
 _lib = None
 
@@ -141,6 +141,9 @@ def load():
     lib.mr_gp_correct_heading.argtypes = [P(GPModel), P(GPModel), C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double,
                                           C.c_double, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.mr_gp_correct_heading.restype = C.c_int
+    lib.mr_gp_correct_action_2d.argtypes = [P(GPModel), P(GPModel), C.c_void_p, C.c_int64, C.c_double, C.c_double * 2,
+                                            C.c_double * 2, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.mr_gp_correct_action_2d.restype = C.c_int
     lib.mr_gp_fit.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_double,
                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                               C.c_void_p]

@@ -13,6 +13,7 @@
 //   It runs on the FP64 tensor pipe (mma.sync m8n8k4 f64 = DMMA; tcgen05 has no fp64 kind),
 //   128x128 CTA tiles, cp.async double-buffered shared-memory staging, fused square-sum epilogue.
 #include <cuda_runtime.h>
+#include <math_constants.h>
 
 #include "mr_actor.cuh"
 #include "mr_actor_tc.cuh"
@@ -475,6 +476,171 @@ gp_correct_heading_cheb_kernel(const double* __restrict__ vd, int64_t n, Heading
     if (nfev_out) nfev_out[row] = num;
 }
 
+// ---- LearningModule2D.predict: batched box-constrained least squares over (alpha, f) --------
+// Learning_module_2d.py:11-25 minimises (a0 f)^2 + (muX - vd0)^2 + 2 a0 f cos(alpha) (muX - vd0) + (muY - vd1)^2 + ...,
+// which is exactly |r|^2 for r(alpha, f) = a0 f (cos alpha, sin alpha) + (muX, muY)(alpha, f) - vd.  One warp per desired
+// velocity; one PASS evaluates, at a trial point, both GP means with their gradients and Hessians (lanes stride the
+// training points, xor-shuffle reduction: 6 sums per GP), so r, its Jacobian J and the Hessian of |r|^2 / 2,
+// H = J^T J + r0 d2(r0) + r1 d2(r1), come out of one pass.  The solver is a projected Newton method with
+// Levenberg-Marquardt damping (Nielsen's update), held redundantly by all lanes:
+//   - a coordinate on a bound whose gradient g = J^T r points out of the box is held fixed; the damped 2x2 (or 1x1)
+//     system is solved on the free coordinates and the trial point is clipped to the box;
+//   - a trial is accepted if |r|^2 decreases; each trial is one pass;
+//   - converged (status 0) when the projected gradient |x - clip(x - g)|_inf <= kAction2dGtol (1 + |vd|^2), or the
+//     next step is at rounding level; kAction2dMaxPass passes -> status 1 with the best point so far;
+//   - a non-finite vd, or non-finite means at the start point -> x = NaN, status 2.
+// The curvature terms r.d2r matter where the minimum is not a root (f on a bound, low speeds): with J^T J alone the
+// solver converges only linearly there (30-60 passes against 7-20 with them in a numpy model of this solver).
+// The exponentials use the table form the staged mr_gp_predict kernel uses, in the same order per lane.
+constexpr double kAction2dGtol = 1e-12;
+constexpr int kAction2dMaxPass = 64;
+
+struct GpMoments2 { double m, s0, s1, s00, s01, s11; };   // sum a_j k_j (1, s, s s^T) with s_j = q / l - X_j / l
+
+__device__ __forceinline__ void gp_moments_2d_warp(double q0, double q1, const double* __restrict__ xsx,
+                                                   const double* __restrict__ ax, double lsx, const double* __restrict__ xsy,
+                                                   const double* __restrict__ ay, double lsy, int n_train, int lane,
+                                                   const double* __restrict__ tab, GpMoments2& mx, GpMoments2& my) {
+    const double px0 = q0 / lsx, px1 = q1 / lsx, py0 = q0 / lsy, py1 = q1 / lsy;
+    double v[12];
+#pragma unroll
+    for (int i = 0; i < 12; ++i) v[i] = 0.0;
+    for (int j = lane; j < n_train; j += 32) {
+        const double dx0 = px0 - xsx[2 * j], dx1 = px1 - xsx[2 * j + 1];
+        const double dy0 = py0 - xsy[2 * j], dy1 = py1 - xsy[2 * j + 1];
+        double d2x = dx0 * dx0, d2y = dy0 * dy0;
+        d2x = fma(dx1, dx1, d2x);
+        d2y = fma(dy1, dy1, d2y);
+        const double kx = exp_neg_tab(-0.5 * d2x, tab), ky = exp_neg_tab(-0.5 * d2y, tab);
+        const double ajx = ax[j], ajy = ay[j];
+        v[0] = fma(kx, ajx, v[0]);
+        v[6] = fma(ky, ajy, v[6]);
+        const double wx = kx * ajx, wy = ky * ajy;
+        const double wx0 = wx * dx0, wy0 = wy * dy0, wx1 = wx * dx1, wy1 = wy * dy1;
+        v[1] += wx0; v[2] += wx1; v[3] = fma(wx0, dx0, v[3]); v[4] = fma(wx0, dx1, v[4]); v[5] = fma(wx1, dx1, v[5]);
+        v[7] += wy0; v[8] += wy1; v[9] = fma(wy0, dy0, v[9]); v[10] = fma(wy0, dy1, v[10]); v[11] = fma(wy1, dy1, v[11]);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1)
+#pragma unroll
+        for (int i = 0; i < 12; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], off);
+    mx = GpMoments2{v[0], v[1], v[2], v[3], v[4], v[5]};
+    my = GpMoments2{v[6], v[7], v[8], v[9], v[10], v[11]};
+}
+
+struct Action2dState { double r0, r1, g0, g1, h00, h01, h11, F; };
+
+// residual, gradient g = J^T r and Hessian H of |r|^2 / 2 at (alpha, f) from the two GPs' moments
+__device__ __forceinline__ Action2dState action_2d_state(double alpha, double f, double vd0, double vd1, double a0,
+                                                         const GpMoments2& mx, double lsx, const GpMoments2& my, double lsy) {
+    double sa, ca;
+    sincos(alpha, &sa, &ca);
+    const double a0f = a0 * f;
+    Action2dState st;
+    st.r0 = fma(a0f, ca, mx.m) - vd0;
+    st.r1 = fma(a0f, sa, my.m) - vd1;
+    // d mu / d q = -S / l ;  d2 mu / dq dq^T = (S2 - mu I) / l^2
+    const double ix = 1.0 / lsx, iy = 1.0 / lsy;
+    const double j00 = -a0f * sa - mx.s0 * ix, j01 = a0 * ca - mx.s1 * ix;
+    const double j10 = a0f * ca - my.s0 * iy, j11 = a0 * sa - my.s1 * iy;
+    st.g0 = j00 * st.r0 + j10 * st.r1;
+    st.g1 = j01 * st.r0 + j11 * st.r1;
+    const double cx = st.r0 * ix * ix, cy = st.r1 * iy * iy;
+    const double c00 = cx * (mx.s00 - mx.m) + cy * (my.s00 - my.m) - a0f * (st.r0 * ca + st.r1 * sa);
+    const double c01 = cx * mx.s01 + cy * my.s01 + a0 * (st.r1 * ca - st.r0 * sa);
+    const double c11 = cx * (mx.s11 - mx.m) + cy * (my.s11 - my.m);
+    st.h00 = j00 * j00 + j10 * j10 + c00;
+    st.h01 = j00 * j01 + j10 * j11 + c01;
+    st.h11 = j01 * j01 + j11 * j11 + c11;
+    st.F = st.r0 * st.r0 + st.r1 * st.r1;
+    return st;
+}
+
+__global__ void __launch_bounds__(256)
+gp_correct_action_2d_kernel(const double* __restrict__ vd, int64_t n, double a0, const double* __restrict__ xsx,
+                            const double* __restrict__ ax, double lsx, const double* __restrict__ xsy,
+                            const double* __restrict__ ay, double lsy, int n_train, double lo0, double lo1, double hi0,
+                            double hi1, double* __restrict__ x_out, int32_t* __restrict__ iters_out,
+                            uint8_t* __restrict__ status_out) {
+    __shared__ double s_tab[64];
+    exp_table_init(s_tab);
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (row >= n) return;
+    const double vd0 = vd[2 * row], vd1 = vd[2 * row + 1];
+    auto clip0 = [&](double v) { return fmin(fmax(v, lo0), hi0); };
+    auto clip1 = [&](double v) { return fmin(fmax(v, lo1), hi1); };
+    auto eval = [&](double alpha, double f) {
+        GpMoments2 mx, my;
+        gp_moments_2d_warp(alpha, f, xsx, ax, lsx, xsy, ay, lsy, n_train, lane, s_tab, mx, my);
+        return action_2d_state(alpha, f, vd0, vd1, a0, mx, lsx, my, lsy);
+    };
+    double x0 = CUDART_NAN, x1 = CUDART_NAN;
+    int passes = 0, status = 2;
+    if (isfinite(vd0) && isfinite(vd1)) {
+        // Learning_module_2d.py:229-230 (_desired), clipped into the box as L-BFGS-B clips its x0
+        x0 = clip0(atan2(vd1, vd0));
+        x1 = clip1(sqrt(fma(vd1, vd1, vd0 * vd0)) / a0);
+        Action2dState s = eval(x0, x1);
+        passes = 1;
+        if (!isfinite(s.F)) {
+            x0 = x1 = CUDART_NAN;
+        } else {
+            const double gtol = kAction2dGtol * (1.0 + fma(vd1, vd1, vd0 * vd0));
+            const double step_eps = 0x1p-50;
+            double mu = 1e-3 * fmax(fmax(fabs(s.h00), fabs(s.h11)), 1e-300), nu = 2.0;
+            status = -1;
+            while (status < 0) {
+                const double pg = fmax(fabs(x0 - clip0(x0 - s.g0)), fabs(x1 - clip1(x1 - s.g1)));
+                if (pg <= gtol) { status = 0; break; }
+                const bool free0 = !((x0 <= lo0 && s.g0 > 0.0) || (x0 >= hi0 && s.g0 < 0.0));
+                const bool free1 = !((x1 <= lo1 && s.g1 > 0.0) || (x1 >= hi1 && s.g1 < 0.0));
+                for (;;) {                                         // damped trials until one is accepted
+                    if (!(mu <= 1e300)) { status = 1; break; }    // only a non-finite Hessian gets here
+                    double d0 = 0.0, d1 = 0.0;
+                    const double a00 = s.h00 + mu, a11 = s.h11 + mu;
+                    if (free0 && free1) {
+                        const double det = a00 * a11 - s.h01 * s.h01;
+                        if (!(det > 0.0 && a00 > 0.0)) { mu *= nu; nu *= 2.0; continue; }   // not positive definite yet
+                        d0 = (s.h01 * s.g1 - a11 * s.g0) / det;
+                        d1 = (s.h01 * s.g0 - a00 * s.g1) / det;
+                    } else if (free0) {
+                        if (!(a00 > 0.0)) { mu *= nu; nu *= 2.0; continue; }
+                        d0 = -s.g0 / a00;
+                    } else {                                       // pg > 0 leaves at least one coordinate free
+                        if (!(a11 > 0.0)) { mu *= nu; nu *= 2.0; continue; }
+                        d1 = -s.g1 / a11;
+                    }
+                    const double t0 = clip0(x0 + d0), t1 = clip1(x1 + d1);
+                    const double h0 = t0 - x0, h1 = t1 - x1;
+                    if (fabs(h0) <= step_eps * (1.0 + fabs(x0)) && fabs(h1) <= step_eps * (1.0 + fabs(x1))) { status = 0; break; }
+                    if (passes >= kAction2dMaxPass) { status = 1; break; }
+                    const Action2dState t = eval(t0, t1);
+                    ++passes;
+                    if (t.F < s.F) {
+                        // gain ratio against the quadratic model of |r|^2 / 2 along the (clipped) step
+                        const double pred = -(s.g0 * h0 + s.g1 * h1) - 0.5 * (h0 * h0 * s.h00 + 2.0 * h0 * h1 * s.h01 + h1 * h1 * s.h11);
+                        const double rho = pred > 0.0 ? 0.5 * (s.F - t.F) / pred : 0.0;
+                        const double c = 2.0 * rho - 1.0;
+                        mu *= fmax(1.0 / 3.0, 1.0 - c * c * c);
+                        nu = 2.0;
+                        x0 = t0; x1 = t1; s = t;
+                        break;
+                    }
+                    mu *= nu; nu *= 2.0;                            // rejected (also when t.F is NaN)
+                }
+            }
+        }
+    }
+    if (lane == 0) {
+        x_out[2 * row] = x0;
+        x_out[2 * row + 1] = x1;
+        if (iters_out) iters_out[row] = passes;
+        if (status_out) status_out[row] = (uint8_t)status;
+    }
+}
+
 static bool fused_spectral_disabled() {          // MR_GP_FUSED=0: keep the two-kernel path for the spectral form (A/B measurements)
     static const bool off = [] { const char* e = getenv("MR_GP_FUSED"); return e && e[0] == '0'; }();
     return off;
@@ -647,6 +813,34 @@ int mr_gp_correct_heading_cheb(const double* coef_x, const double* coef_y, int32
     gp_correct_heading_cheb_kernel<<<blocks, 128, smem, (cudaStream_t)stream>>>(vd, n, hp, coef_x, coef_y, n_coef, -3.141592653589793,
                                                                                3.141592653589793, 1e-5, 500, alpha_out, nfev_out);
     return check_launch("mr_gp_correct_heading_cheb");
+}
+
+int mr_gp_correct_action_2d(const mr_gp_model* gpx, const mr_gp_model* gpy, const double* vd, int64_t n, double a0,
+                            const double lo[2], const double hi[2], double* x_out, int32_t* iters_out, uint8_t* status_out,
+                            void* stream) {
+    mr::NvtxRange nvtx_range("mr_gp_correct_action_2d");
+    using namespace mr;
+    if (!gpx || !gpy || !gpx->x_train_scaled || !gpy->x_train_scaled || !gpx->alpha || !gpy->alpha)
+        return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: null model");
+    if (gpx->dim != 2 || gpy->dim != 2) return fail(MR_ERR_UNSUPPORTED, "mr_gp_correct_action_2d: (alpha, f) GPs have dim 2");
+    if (gpx->n_pad != gpy->n_pad || gpx->n_train != gpy->n_train)
+        return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: the two GPs must share their training inputs");
+    if (gpx->n_train <= 0 || gpx->n_train > gpx->n_pad || !(gpx->length_scale > 0) || !(gpy->length_scale > 0))
+        return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: bad n_train / length_scale");
+    if (n < 0) return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: bad n");
+    if (n == 0) return MR_OK;
+    if (!vd || !x_out) return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: null vd/x_out");
+    if (!lo || !hi) return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: null bounds");
+    for (int c = 0; c < 2; ++c)
+        if (!std::isfinite(lo[c]) || !std::isfinite(hi[c]) || !(lo[c] < hi[c]))
+            return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: bounds must be finite with lo < hi");
+    if (!std::isfinite(a0) || !(a0 > 0)) return fail(MR_ERR_ARG, "mr_gp_correct_action_2d: a0 must be finite and > 0");
+    const int threads = 256;
+    const unsigned blocks = (unsigned)((n * 32 + threads - 1) / threads);
+    gp_correct_action_2d_kernel<<<blocks, threads, 0, (cudaStream_t)stream>>>(
+        vd, n, a0, gpx->x_train_scaled, gpx->alpha, gpx->length_scale, gpy->x_train_scaled, gpy->alpha, gpy->length_scale,
+        gpx->n_train, lo[0], lo[1], hi[0], hi[1], x_out, iters_out, status_out);
+    return check_launch("mr_gp_correct_action_2d");
 }
 
 int32_t mr_actor_param_count(void) { return mr::kActorParams; }

@@ -17,6 +17,8 @@ from .gp import DeviceGP
 
 
 class LearningModule2D:
+    BOUNDS = ((-np.pi, np.pi), (0, 5))     # the (alpha, f) box of the corrected action, Learning_module_2d.py:258
+
     def __init__(self, device="cuda", fit="device"):
         if fit == "device":
             from .gpr import DeviceGPR
@@ -121,12 +123,41 @@ class LearningModule2D:
         return (a0 * freq) ** 2 + (mux - vd[0]) ** 2 + 2 * a0 * freq * np.cos(alpha) * (mux - vd[0]) \
             + (muy - vd[1]) ** 2 + 2 * a0 * freq * np.sin(alpha) * (muy - vd[1])
 
+    def predict_batch(self, vd, return_info=False):
+        """LearningModule2D.predict for vd [N, 2] (array or device tensor) in one device call (mr_gp_correct_action_2d):
+        the minimiser over (alpha, f) in BOUNDS of the reference's objective, which equals |r|^2 for
+        r = a0 f (cos alpha, sin alpha) + (muX, muY)(alpha, f) - vd, found by a projected Newton / Levenberg-Marquardt
+        search with both GP means, gradients and Hessians evaluated on the device; then the posterior at the minimiser
+        through gp_batch, the kernels error() uses.
+        Returns (X [N, 2], muX, muY, sigX, sigY) device tensors, plus (iters [N] int32 passes, status [N] uint8) with
+        ``return_info=True``.  Rows whose search did not converge are returned, not raised: status 1 = the 64-pass cap
+        was reached and X is the best point found; status 2 = vd was not finite (or the GP means were not finite at the
+        start point) and X is NaN."""
+        import ctypes as C
+
+        from . import _lib as L
+        dev = torch.device(self.device)
+        vd = torch.as_tensor(vd).to(device=dev, dtype=torch.float64).reshape(-1, 2).contiguous()
+        n = vd.shape[0]
+        X = torch.empty((n, 2), dtype=torch.float64, device=dev)
+        iters = torch.empty(n, dtype=torch.int32, device=dev)
+        status = torch.empty(n, dtype=torch.uint8, device=dev)
+        (lo0, hi0), (lo1, hi1) = self.BOUNDS
+        with torch.cuda.device(dev):
+            rc = L.load().mr_gp_correct_action_2d(C.byref(self._dx._c), C.byref(self._dy._c), vd.data_ptr(), n, float(self.a0),
+                                                  (C.c_double * 2)(lo0, lo1), (C.c_double * 2)(hi0, hi1), X.data_ptr(),
+                                                  iters.data_ptr(), status.data_ptr(),
+                                                  C.c_void_p(torch.cuda.current_stream(dev).cuda_stream))
+        L.check(rc, "mr_gp_correct_action_2d")
+        mx, my, sx, sy = self.gp_batch(X)
+        return (X, mx, my, sx, sy, iters, status) if return_info else (X, mx, my, sx, sy)
+
     def predict(self, vd):
         """Learning_module_2d.py:239-268: scipy minimize over (alpha, f) in [-pi, pi] x [0, 5] from the desired values."""
         from scipy.optimize import minimize
         vd = np.asarray(vd, float).ravel()
         x0 = self._desired(vd)
-        result = minimize(self._objective, x0, args=(vd,), bounds=[(-np.pi, np.pi), (0, 5)])
+        result = minimize(self._objective, x0, args=(vd,), bounds=self.BOUNDS)
         X = np.array(result.x)
         mx, my, sx, sy = (t.cpu().numpy() for t in self.gp_batch(X))
         return X, mx, my, sx, sy
