@@ -13,6 +13,7 @@
  *                       MR_Env.convert_state / end / calculate_reward (MR_env.py:100-152)
  *   mr_env_rollout   <- utils.run_sim           (utils.py:43-61)   open-loop K-step rollout
  *                       RL/MR_ddpg.py:268-311   closed loop with ActorNetwork.predict (:124-149)
+ *   mr_env_rollout_gp_heading <- the GP-corrected run of main.py (vd at :147), open or closed loop, fused
  *   mr_gp_predict    <- LearningModule.error / objective / predict -> sklearn GPR.predict
  *                       (Learning_module.py:10-24,186-224)
  *   mr_gp_correct_heading <- LearningModule.predict's minimize_scalar(objective, 'Bounded')
@@ -79,7 +80,9 @@ enum mr_action_source {
     MR_ACTIONS_TENSOR = 0,      /* actions[K][n][2] */
     MR_ACTIONS_PHILOX = 1,      /* uniform in action_space, generated in-kernel */
     MR_ACTIONS_ACTOR = 2,       /* DDPG actor MLP evaluated in-kernel on the observation */
-    MR_ACTIONS_BROADCAST = 3    /* actions[K][2], the same action for every env (utils.run_sim) */
+    MR_ACTIONS_BROADCAST = 3,   /* actions[K][2], the same action for every env (utils.run_sim) */
+    MR_ACTIONS_GP_HEADING = 4   /* GP-corrected heading control (mr_gp_heading_policy); accepted only by
+                                   mr_env_rollout_gp_heading, mr_env_rollout rejects it */
 };
 
 /* Simulator + env parameters (MR_simulator.py:12-19, MR_env.py:34-63).  Launch scalars. */
@@ -248,6 +251,31 @@ enum { MR_STAT_EPISODES = 0, MR_STAT_SUM_LENGTH = 1, MR_STAT_SUM_REWARD = 2, MR_
 int mr_env_rollout(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
                    const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
                    const mr_step_out* out, void* stream);
+
+/* The GP-corrected heading controller of main.py (:147) run inside the fused rollout.  Per env and step k, with
+ * (x, y) the position at the start of step k:
+ *     vd    = (vx_ref[k] + gain * (x_ref[k] - x),  vy_ref[k] + gain * (y_ref[k] - y))
+ *     alpha = the heading search of mr_gp_correct_heading_cheb for vd (same objective, [-pi, pi], xatol 1e-5, maxfun 500)
+ *     action = (freq, alpha)
+ * Each of the four operations per component is rounded on its own (no fused multiply-add), so the same expression in
+ * torch / numpy gives the same vd bits.  gain = 0 is main.py's open-loop correction (vd = v_ref[k]).  ref is the same for
+ * every env. */
+typedef struct mr_gp_heading_policy {
+    const double* coef_x;  /* [n_coef] Chebyshev series of GP mean X on [-pi, pi] (as for mr_gp_correct_heading_cheb) */
+    const double* coef_y;  /* [n_coef] */
+    int32_t n_coef;        /* 1 .. 4096 */
+    int32_t reserved;
+    double a0, freq, drift_x, drift_y;   /* LearningModule.a0, .freq, .Dx, .Dy */
+    const double* ref;     /* [k_steps][4]: x_ref, y_ref (start of step k), vx_ref, vy_ref */
+    double gain;           /* position feedback, 1/s; 0 = open loop */
+} mr_gp_heading_policy;
+
+/* mr_env_rollout with the actions of mr_gp_heading_policy (io->action_source must be MR_ACTIONS_GP_HEADING; io->actions
+ * and io->actor are ignored).  Every other member of io (recording rows, statistics, reset_init) works as for
+ * mr_env_rollout; traj_actions records (freq, alpha).  Per-env parameter rows are not supported (MR_ERR_UNSUPPORTED). */
+int mr_env_rollout_gp_heading(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                              const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
+                              const mr_gp_heading_policy* pol, const mr_step_out* out, void* stream);
 
 /* ---- Gaussian-process inference (Learning_module.py -> sklearn GPR.predict) ----------
  * The fitted model (GPR.X_train_, alpha_, L_, kernel_ = RBF(length_scale) + WhiteKernel(noise_level))

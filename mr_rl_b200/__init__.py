@@ -5,6 +5,7 @@ Public surface (mirrors the reference's names):
     MR_Env, Simulator             single-env façades with the reference's class surface
     run_sim                       utils.run_sim as one fused rollout launch
     LearningModule, LearningModule2D, DeviceGP, DeviceGPR   GP disturbance model: fit, inference and heading correction on the device
+    HeadingTrackingPolicy         LearningModule.tracking_policy: GP-corrected heading control inside VecMREnv.rollout
     DDPGLearner, ReplayBuffer, OUNoise, ddpg.train   the DDPG learner of RL/MR_ddpg.py on the device
     init_actor / pack_actor / actor_forward   DDPG actor forward for the in-loop policy
     experiment_dict / save_experiment          recorded rollouts in the reference's MRExperiment pickle layout
@@ -17,7 +18,7 @@ from .actor import actor_forward, init_actor, pack_actor  # noqa: F401
 from .ddpg import DDPGLearner, OUNoise, ReplayBuffer  # noqa: F401
 from .gp import DeviceGP  # noqa: F401
 from .gpr import DeviceGPR  # noqa: F401
-from .learning_module import LearningModule  # noqa: F401
+from .learning_module import HeadingTrackingPolicy, LearningModule  # noqa: F401
 from .learning_module_2d import LearningModule2D  # noqa: F401
 from .mr_env import MR_Env, Simulator  # noqa: F401
 from .recording import MRExperiment, experiment_dict, experiment_from_rollout, load_experiment, save_experiment  # noqa: F401

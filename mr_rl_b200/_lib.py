@@ -15,6 +15,7 @@ ABI_VERSION = 2
 MR_F64, MR_F32 = 0, 1
 NOISE_NONE, NOISE_TABLE, NOISE_PHILOX = 0, 1, 2
 ACTIONS_TENSOR, ACTIONS_PHILOX, ACTIONS_ACTOR, ACTIONS_BROADCAST = 0, 1, 2, 3
+ACTIONS_GP_HEADING = 4          # mr_env_rollout_gp_heading only
 REWARD_CONST10, REWARD_SHAPED = 0, 1
 ENV_SOLVER_FAILED, ENV_NONFINITE, ENV_NOISE_OVERFLOW, ENV_ATTEMPT_CAP = 1, 2, 4, 8
 STATS_LEN = 8
@@ -65,6 +66,12 @@ class RolloutIO(C.Structure):
                 ("reset_init", C.c_void_p), ("reset_init_len", C.c_int32), ("reserved", C.c_int32)]
 
 
+class GpHeadingPolicy(C.Structure):
+    _fields_ = [("coef_x", C.c_void_p), ("coef_y", C.c_void_p), ("n_coef", C.c_int32), ("reserved", C.c_int32),
+                ("a0", C.c_double), ("freq", C.c_double), ("drift_x", C.c_double), ("drift_y", C.c_double),
+                ("ref", C.c_void_p), ("gain", C.c_double)]
+
+
 class GPModel(C.Structure):
     _fields_ = [("x_train_scaled", C.c_void_p), ("alpha", C.c_void_p), ("linv", C.c_void_p), ("n_train", C.c_int32),
                 ("n_pad", C.c_int32), ("dim", C.c_int32), ("proj_rows", C.c_int32),
@@ -99,7 +106,8 @@ EXPORTS = ("mr_abi_version", "mr_last_error", "mr_default_params", "mr_fill_time
            "mr_critic_param_count", "mr_replay_add", "mr_ou_noise_add", "mr_ddpg_update", "mr_learn_preprocess",
            "mr_learn_workspace_bytes", "mr_ddpg_workspace_bytes", "mr_replay_sample", "mr_actor_forward_env", "mr_ddpg_gradients", "mr_ddpg_apply", "mr_gp_correct_heading_cheb", "mr_host_pipeline_create", "mr_host_pipeline_destroy", "mr_env_step_host",
            "mr_actor_forward", "mr_set_step_path", "mr_env_reset_ex", "mr_counter_set", "mr_set_actor_path",
-           "mr_host_register", "mr_host_unregister", "mr_philox_normals", "mr_gp_correct_action_2d")
+           "mr_host_register", "mr_host_unregister", "mr_philox_normals", "mr_gp_correct_action_2d",
+           "mr_env_rollout_gp_heading")
 
 _lib = None
 
@@ -136,6 +144,9 @@ def load():
                                 P(StepOut), C.c_void_p]
     lib.mr_env_rollout.argtypes = [P(EnvState), C.c_int64, C.c_int32, P(SimParams), P(Noise), P(TimeTable),
                                    P(RolloutIO), P(StepOut), C.c_void_p]
+    lib.mr_env_rollout_gp_heading.argtypes = [P(EnvState), C.c_int64, C.c_int32, P(SimParams), P(Noise), P(TimeTable),
+                                              P(RolloutIO), P(GpHeadingPolicy), P(StepOut), C.c_void_p]
+    lib.mr_env_rollout_gp_heading.restype = C.c_int
     lib.mr_gp_predict.argtypes = [P(GPModel), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                   C.c_void_p]
     lib.mr_gp_correct_heading.argtypes = [P(GPModel), P(GPModel), C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double,

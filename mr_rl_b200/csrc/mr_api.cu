@@ -1,5 +1,6 @@
 // Exported C ABI of the env path (include/mr_rl_b200.h): argument checks and dispatch to the
 // per-(storage dtype, noise mode) launchers.  No CPU fallback exists: every call launches CUDA.
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -244,8 +245,7 @@ __global__ void philox_normals_kernel(KeysOnly k, uint64_t env_base, uint64_t st
 }
 
 template <class T>
-static int do_rollout(const mr_env_state& st, int64_t n, const Params& p, const mr_noise* nz, const TimeView& tv,
-                      const mr_rollout_io& io, const mr_step_out* out, cudaStream_t s) {
+static RolloutView<T> rollout_view(const mr_rollout_io& io) {
     RolloutView<T> rv;
     rv.actions = (const T*)io.actions; rv.actor = io.actor; rv.traj_xy = (T*)io.traj_xy;
     rv.traj_sp = (T*)io.traj_state_prime; rv.traj_done = io.traj_done; rv.stats = io.stats;
@@ -253,6 +253,13 @@ static int do_rollout(const mr_env_state& st, int64_t n, const Params& p, const 
     rv.traj_episode = io.traj_episode; rv.traj_step = io.traj_step; rv.episode_counter = io.episode_counter;
     rv.reset_init = (const T*)io.reset_init; rv.reset_init_len = io.reset_init_len;
     rv.k_steps = io.k_steps; rv.action_source = io.action_source;
+    return rv;
+}
+
+template <class T>
+static int do_rollout(const mr_env_state& st, int64_t n, const Params& p, const mr_noise* nz, const TimeView& tv,
+                      const mr_rollout_io& io, const mr_step_out* out, cudaStream_t s) {
+    const RolloutView<T> rv = rollout_view<T>(io);
     const StateView<T> sv = state_view<T>(st);
     const OutView<T> ov = out_view<T>(out, n);
     const NoiseView nv = noise_view(nz, n);
@@ -261,6 +268,32 @@ static int do_rollout(const mr_env_state& st, int64_t n, const Params& p, const 
         case MR_NOISE_PHILOX: return launch_rollout<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, s);
         default: return launch_rollout<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, s);
     }
+}
+
+template <class T>
+static int do_rollout_gp(const mr_env_state& st, int64_t n, const Params& p, const mr_noise* nz, const TimeView& tv,
+                         const mr_rollout_io& io, const GpHeadingView& gh, const mr_step_out* out, cudaStream_t s) {
+    const RolloutView<T> rv = rollout_view<T>(io);
+    const StateView<T> sv = state_view<T>(st);
+    const OutView<T> ov = out_view<T>(out, n);
+    const NoiseView nv = noise_view(nz, n);
+    switch (nz ? nz->mode : MR_NOISE_NONE) {
+        case MR_NOISE_TABLE: return launch_rollout_gp<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, gh, s);
+        case MR_NOISE_PHILOX: return launch_rollout_gp<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, gh, s);
+        default: return launch_rollout_gp<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, gh, s);
+    }
+}
+
+// the checks of mr_env_rollout that do not depend on the action source
+static int check_rollout(const char* fn, const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                         const mr_noise* nz, const mr_rollout_io* io, const mr_step_out* out) {
+    int rc = check_common(fn, st, n, dtype, p, nz);
+    if (rc) return rc;
+    if (!io || io->k_steps < 0) return fail(MR_ERR_ARG, "%s: bad io", fn);
+    if (p->auto_reset && nz == nullptr) return fail(MR_ERR_ARG, "%s: auto_reset needs mr_noise (seed) for the init sampler", fn);
+    if (out && out->out_f32) return fail(MR_ERR_UNSUPPORTED, "%s: float32 output rows are a step option", fn);
+    if (io->reset_init && io->reset_init_len <= 0) return fail(MR_ERR_ARG, "%s: reset_init needs reset_init_len > 0", fn);
+    return MR_OK;
 }
 
 }  // namespace mr
@@ -557,3 +590,37 @@ int mr_env_rollout(const mr_env_state* st, int64_t n, int32_t dtype, const mr_si
 }
 
 }  // extern "C"
+
+extern "C" int mr_env_rollout_gp_heading(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                                         const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
+                                         const mr_gp_heading_policy* pol, const mr_step_out* out, void* stream) {
+    mr::NvtxRange nvtx_range("mr_env_rollout_gp_heading");
+    using mr::fail;
+    const char* fn = "mr_env_rollout_gp_heading";
+    int rc = mr::check_rollout(fn, st, n, dtype, p, nz, io, out);
+    if (rc) return rc;
+    if (io->action_source != MR_ACTIONS_GP_HEADING)
+        return fail(MR_ERR_ARG, "%s: io->action_source must be MR_ACTIONS_GP_HEADING (%d), got %d", fn, MR_ACTIONS_GP_HEADING,
+                    io->action_source);
+    if (!pol) return fail(MR_ERR_ARG, "%s: null policy", fn);
+    if (!pol->coef_x || !pol->coef_y) return fail(MR_ERR_ARG, "%s: null coefficients", fn);
+    if (!pol->ref) return fail(MR_ERR_ARG, "%s: null ref", fn);
+    if (pol->n_coef < 1 || pol->n_coef > 4096) return fail(MR_ERR_ARG, "%s: need 1 <= n_coef <= 4096", fn);
+    for (double v : {pol->a0, pol->freq, pol->drift_x, pol->drift_y, pol->gain})
+        if (!std::isfinite(v)) return fail(MR_ERR_ARG, "%s: a0, freq, drift_x, drift_y and gain must be finite", fn);
+    if (st->a0) return fail(MR_ERR_UNSUPPORTED, "%s: the GP heading policy does not take per-env parameter rows", fn);
+    if (n == 0 || io->k_steps == 0) return MR_OK;
+    if (!tt || !tt->t || tt->len < 2) return fail(MR_ERR_ARG, "%s: time table missing", fn);
+    const mr::Params pp = mr::to_params(*p, nz);
+    const mr::TimeView tv{tt->t, tt->len};
+    mr::GpHeadingView gh;
+    gh.coef_x = pol->coef_x; gh.coef_y = pol->coef_y; gh.ref = pol->ref;
+    gh.a0f = pol->a0 * pol->freq;                           // as mr_gp_correct_heading_cheb forms it
+    gh.dx = pol->drift_x; gh.dy = pol->drift_y;
+    gh.freq = pol->freq; gh.gain = pol->gain;
+    gh.lo = -3.141592653589793; gh.hi = 3.141592653589793; gh.xatol = 1e-5;
+    gh.n_coef = pol->n_coef; gh.maxfun = 500;
+    cudaStream_t s = (cudaStream_t)stream;
+    return dtype == MR_F64 ? mr::do_rollout_gp<double>(*st, n, pp, nz, tv, *io, gh, out, s)
+                           : mr::do_rollout_gp<float>(*st, n, pp, nz, tv, *io, gh, out, s);
+}

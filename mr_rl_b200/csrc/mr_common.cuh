@@ -244,4 +244,19 @@ template <class T, int MODE>
 int launch_rollout(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
                    const TimeView& tv, const Params& p, int64_t n, cudaStream_t s);
 
+// The GP-corrected heading policy of the fused rollout (mr_gp_heading_policy): per env and step k the desired velocity
+// vd = v_ref[k] + gain (p_ref[k] - p), then the heading search of gp_correct_heading_cheb_kernel on [lo, hi].
+struct GpHeadingView {
+    const double* coef_x;      // [n_coef] Chebyshev series of the two GP means on [lo, hi]
+    const double* coef_y;
+    const double* ref;         // [K][4] x_ref, y_ref, vx_ref, vy_ref
+    double a0f, dx, dy;        // HeadingProblem
+    double freq, gain;
+    double lo, hi, xatol;      // search interval and tolerance, passed at run time as the standalone kernel takes them
+    int n_coef, maxfun;
+};
+template <class T, int MODE>
+int launch_rollout_gp(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
+                      const TimeView& tv, const Params& p, int64_t n, const GpHeadingView& gh, cudaStream_t s);
+
 }  // namespace mr

@@ -16,6 +16,32 @@ import torch
 from .gp import DeviceGP
 
 
+class HeadingTrackingPolicy:
+    """The GP-corrected heading controller as an in-kernel policy of ``VecMREnv.rollout`` (``LearningModule.tracking_policy``).
+
+    Per env and step k, from the position p at the start of the step: vd = ref[k, 2:] + gain * (ref[k, :2] - p), then the
+    heading search of ``LearningModule.predict_batch`` for vd, action (freq, alpha).  Every operation of vd is rounded on its
+    own, so that same torch expression gives the same bits.  gain = 0 is the open-loop correction of main.py (vd = v_ref)."""
+
+    def __init__(self, cheb, a0, freq, Dx, Dy, ref, gain):
+        self.cheb = cheb                     # [2, n_coef] verified Chebyshev series of the two GP means on [-pi, pi]
+        self.a0, self.freq, self.Dx, self.Dy = float(a0), float(freq), float(Dx), float(Dy)
+        self.ref = ref                       # [K, 4] fp64: x_ref, y_ref (start of step k), vx_ref, vy_ref
+        self.gain = float(gain)
+
+    @property
+    def k_steps(self):
+        return self.ref.shape[0]
+
+    def c_policy(self, device):
+        """The mr_gp_heading_policy struct for a launch on ``device`` and the tensors it points into (keep them alive)."""
+        from . import _lib as L
+        cheb, ref = self.cheb.to(device).contiguous(), self.ref.to(device).contiguous()
+        pol = L.GpHeadingPolicy(cheb[0].data_ptr(), cheb[1].data_ptr(), cheb.shape[1], 0, self.a0, self.freq, self.Dx,
+                                self.Dy, ref.data_ptr(), self.gain)
+        return pol, (cheb, ref)
+
+
 class LearningModule:
     spectral_variance = True     # evaluate GP variances through the low-rank spectral projection when it is exact to 1e-9
     heading_surrogate = True     # search corrected headings on verified Chebyshev interpolants of the two GP means
@@ -252,6 +278,21 @@ class LearningModule:
             L.check(rc, "mr_gp_correct_heading")
         mx, my, sx, sy = self.gp_batch(alpha, True)
         return (alpha, mx, my, sx, sy, nfev) if return_nfev else (alpha, mx, my, sx, sy)
+
+    def tracking_policy(self, ref, gain=0.0):
+        """The GP-corrected heading controller for ``VecMREnv.rollout(policy=...)``: ref [K, 4] holds, per control step k,
+        the desired position at the start of the step and the desired velocity during it (x_ref, y_ref, vx_ref, vy_ref),
+        the same for every env; gain (1/s) feeds the position error back into the desired velocity, 0 = open loop.
+        Needs the Chebyshev heading surrogate of this model (built and verified by ``upload``)."""
+        if getattr(self, "_cheb", None) is None:
+            raise ValueError("tracking_policy needs the verified Chebyshev heading surrogate, which this model does not have; "
+                             "compose the controller from predict_batch + VecMREnv.step instead")
+        ref = torch.as_tensor(ref).to(device=self.device, dtype=torch.float64).contiguous()
+        if ref.dim() != 2 or ref.shape[1] != 4 or ref.shape[0] < 1:
+            raise ValueError(f"ref must be [K, 4] (x_ref, y_ref, vx_ref, vy_ref), got {tuple(ref.shape)}")
+        if not bool(torch.isfinite(ref).all()):
+            raise ValueError("ref must be finite")
+        return HeadingTrackingPolicy(self._cheb, self.a0, self.freq, self.Dx, self.Dy, ref, gain)
 
     def predict(self, vd):
         """Learning_module.py:198-224: bounded scalar minimisation of the objective over alpha, then the

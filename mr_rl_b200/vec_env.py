@@ -16,6 +16,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
+from .learning_module import HeadingTrackingPolicy
 from .spaces import Box
 
 _DT = {torch.float64: L.MR_F64, torch.float32: L.MR_F32}
@@ -529,7 +530,9 @@ class VecMREnv:
         actions : [K, N, 2] per-env actions, or [K, 2] / [K, >=2] one action row for every env
                   (what utils.run_sim does), or None with ``policy``:
         policy  : "random" -> U[0,20) x U[0,2pi) generated in-kernel (Philox);
-                  a packed float32 actor tensor (see actor.pack_actor) -> DDPG actor in the loop.
+                  a packed float32 actor tensor (see actor.pack_actor) -> DDPG actor in the loop;
+                  a ``LearningModule.tracking_policy(ref, gain)`` -> GP-corrected heading control in the loop
+                  (``k_steps`` defaults to the K rows of its ``ref``; per-env parameter rows are not supported).
         record_episodes : per-episode logging on the device (what MRExperiment.new_iter / new_transition record,
                   MR_data.py:27-57): adds ``actions_traj`` [K,N,2], ``rew_traj`` [K,N], ``reset_xy`` [K,2,N] (start of the
                   episode that follows a terminal step, with auto_reset), ``episode`` / ``step`` [K,N] int32 keys and
@@ -546,6 +549,7 @@ class VecMREnv:
         n = self.num_envs
         io = L.RolloutIO()
         keep = []
+        gp_pol = None
         if actions is not None:
             a = torch.as_tensor(actions) if not torch.is_tensor(actions) else actions
             a = a.to(device=self.device, dtype=self.dtype)
@@ -571,6 +575,13 @@ class VecMREnv:
             io.actor = w.data_ptr()
             keep.append(w)
             k = int(k_steps)
+        elif isinstance(policy, HeadingTrackingPolicy):
+            k = policy.k_steps if k_steps is None else int(k_steps)
+            if k > policy.k_steps:
+                raise ValueError(f"k_steps = {k} exceeds the {policy.k_steps} rows of the policy's ref")
+            io.action_source = L.ACTIONS_GP_HEADING
+            gp_pol, tensors = policy.c_policy(self.device)
+            keep.extend(tensors)
         else:
             raise ValueError("give actions or policy")
         io.k_steps = k
@@ -610,9 +621,15 @@ class VecMREnv:
         if accumulate_stats:
             io.stats = self._stats.data_ptr()
         nz = self._noise_for(self.params.noise_var)
-        rc = self.lib.mr_env_rollout(C.byref(self._c_state), n, self._dt, C.byref(self.params), C.byref(nz),
-                                     C.byref(self._c_tt), C.byref(io), C.byref(self._c_out), self._stream())
-        L.check(rc, "mr_env_rollout")
+        if gp_pol is not None:
+            rc = self.lib.mr_env_rollout_gp_heading(C.byref(self._c_state), n, self._dt, C.byref(self.params), C.byref(nz),
+                                                    C.byref(self._c_tt), C.byref(io), C.byref(gp_pol), C.byref(self._c_out),
+                                                    self._stream())
+            L.check(rc, "mr_env_rollout_gp_heading")
+        else:
+            rc = self.lib.mr_env_rollout(C.byref(self._c_state), n, self._dt, C.byref(self.params), C.byref(nz),
+                                         C.byref(self._c_tt), C.byref(io), C.byref(self._c_out), self._stream())
+            L.check(rc, "mr_env_rollout")
         self.kernel_launches += 1
         self._step_index += k
         res.update(obs=self.obs, rew=self._rew[:n], done=self._done[:n])
