@@ -21,6 +21,7 @@
  *   mr_gp_correct_action_2d <- LearningModule2D.predict's minimize over (alpha, f)  (Learning_module_2d.py:239-268)
  *   mr_actor_forward <- ActorNetwork.predict    (RL/MR_ddpg.py:124-149)
  *   mr_ddpg_update, mr_replay_add, mr_ou_noise_add <- the learner of RL/MR_ddpg.py (:16-78, :163-231, :285-305)
+ *   mr_env_rollout_ddpg_collect <- its acting loop (:268-284: predict + OU noise, env.step, replay add), fused
  *   mr_learn_preprocess <- LearningModule.estimateDisturbance / learn up to the fit (Learning_module.py:46-59, :63-120)
  *   mr_gp_fit        <- GaussianProcessRegressor.fit at given hyper-parameters: K, cholesky, alpha_, L^-1,
  *                       log marginal likelihood  (Learning_module.py:122-123; the optimiser stays on the host)
@@ -464,6 +465,31 @@ int mr_replay_add(const mr_replay* rb, int64_t head, const void* obs, int64_t ob
  * restart from 0 first (OUNoise.reset). */
 int mr_ou_noise_add(double* ou_state, void* actions, const uint8_t* reset_mask, int64_t n, int32_t dtype, double theta, double mu,
                     double sigma, double dt, uint64_t seed, uint64_t counter, uint64_t env_base, void* stream);
+
+/* Experience collection of the DDPG acting loop (:268-284) inside the fused rollout. */
+typedef struct mr_ddpg_collect {
+    double* ou_state;                 /* [n][2] in/out, as mr_ou_noise_add */
+    double ou_theta, ou_mu, ou_sigma, ou_dt;
+    uint64_t ou_seed, ou_counter, ou_env_base;   /* step k draws OU sample ou_counter + k */
+    mr_replay ring;
+    int64_t head;                     /* slot of transition (k = 0, i = 0) */
+} mr_ddpg_collect;
+
+/* mr_env_rollout with the in-kernel actor (io->action_source must be MR_ACTIONS_ACTOR, io->actor the weights) that
+ * also does what K rounds of mr_actor_forward_env -> mr_ou_noise_add -> mr_env_step -> mr_replay_add do.  Per env i
+ * and step k: a = mu(s_k) + the next OU sample (counter ou_counter + k), rounded to the storage dtype; the env steps
+ * with a; the transition (s_k, a, r, done, s2_k) goes to ring slot (head + k n + i) % capacity as float32 rows.  s_0
+ * is the env's observation rows (out->obs, which must be given); s2_k is the observation after the step, after an
+ * auto reset the new episode's first one.  Transitions that a later one of the same launch overwrites are not
+ * written (k n + i < K n - capacity), so the ring ends as after the K sequential adds.  With float32 storage the
+ * state is rounded to float32 after every step, as the single-step kernel stores it, so the results equal the
+ * composed loop's bit for bit on the 3xTF32 actor path (mr_set_actor_path(2)); the default 3xFP16 path is supported,
+ * the CUDA-core path returns MR_ERR_UNSUPPORTED.  Every other io member works as for mr_env_rollout.  The caller
+ * advances head by K n (mod capacity), count to min(count + K n, capacity) and the OU counter by K.  Requires
+ * n <= capacity and 0 <= head < capacity; per-env parameter rows are not supported (MR_ERR_UNSUPPORTED). */
+int mr_env_rollout_ddpg_collect(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p, const mr_noise* nz,
+                                const mr_time_table* tt, const mr_rollout_io* io, const mr_ddpg_collect* c,
+                                const mr_step_out* out, void* stream);
 
 /* One pass of the reference's update block (:285-305) in ONE launch: minibatch (rows `indices[batch]`, or if NULL a
  * uniform sample without replacement from the first `count` ring rows, Philox keyed by (seed; update_index)),

@@ -7,6 +7,7 @@ Public surface (mirrors the reference's names):
     LearningModule, LearningModule2D, DeviceGP, DeviceGPR   GP disturbance model: fit, inference and heading correction on the device
     HeadingTrackingPolicy         LearningModule.tracking_policy: GP-corrected heading control inside VecMREnv.rollout
     DDPGLearner, ReplayBuffer, OUNoise, ddpg.train   the DDPG learner of RL/MR_ddpg.py on the device
+    ddpg.collect                  its acting loop (actor + OU noise + env step + replay add) fused into one rollout launch
     init_actor / pack_actor / actor_forward   DDPG actor forward for the in-loop policy
     experiment_dict / save_experiment          recorded rollouts in the reference's MRExperiment pickle layout
 

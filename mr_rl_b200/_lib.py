@@ -93,6 +93,12 @@ class Replay(C.Structure):
                 ("capacity", C.c_int64)]
 
 
+class DDPGCollect(C.Structure):
+    _fields_ = [("ou_state", C.c_void_p), ("ou_theta", C.c_double), ("ou_mu", C.c_double), ("ou_sigma", C.c_double),
+                ("ou_dt", C.c_double), ("ou_seed", C.c_uint64), ("ou_counter", C.c_uint64), ("ou_env_base", C.c_uint64),
+                ("ring", Replay), ("head", C.c_int64)]
+
+
 class DDPGHyper(C.Structure):
     _fields_ = [("gamma", C.c_double), ("tau", C.c_double), ("lr_actor", C.c_double), ("lr_critic", C.c_double),
                 ("action_bound", C.c_double * 2), ("adam_beta1", C.c_double), ("adam_beta2", C.c_double), ("adam_eps", C.c_double)]
@@ -107,7 +113,7 @@ EXPORTS = ("mr_abi_version", "mr_last_error", "mr_default_params", "mr_fill_time
            "mr_learn_workspace_bytes", "mr_ddpg_workspace_bytes", "mr_replay_sample", "mr_actor_forward_env", "mr_ddpg_gradients", "mr_ddpg_apply", "mr_gp_correct_heading_cheb", "mr_host_pipeline_create", "mr_host_pipeline_destroy", "mr_env_step_host",
            "mr_actor_forward", "mr_set_step_path", "mr_env_reset_ex", "mr_counter_set", "mr_set_actor_path",
            "mr_host_register", "mr_host_unregister", "mr_philox_normals", "mr_gp_correct_action_2d",
-           "mr_env_rollout_gp_heading")
+           "mr_env_rollout_gp_heading", "mr_env_rollout_ddpg_collect")
 
 _lib = None
 
@@ -147,6 +153,9 @@ def load():
     lib.mr_env_rollout_gp_heading.argtypes = [P(EnvState), C.c_int64, C.c_int32, P(SimParams), P(Noise), P(TimeTable),
                                               P(RolloutIO), P(GpHeadingPolicy), P(StepOut), C.c_void_p]
     lib.mr_env_rollout_gp_heading.restype = C.c_int
+    lib.mr_env_rollout_ddpg_collect.argtypes = [P(EnvState), C.c_int64, C.c_int32, P(SimParams), P(Noise), P(TimeTable),
+                                                P(RolloutIO), P(DDPGCollect), P(StepOut), C.c_void_p]
+    lib.mr_env_rollout_ddpg_collect.restype = C.c_int
     lib.mr_gp_predict.argtypes = [P(GPModel), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                   C.c_void_p]
     lib.mr_gp_correct_heading.argtypes = [P(GPModel), P(GPModel), C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double,

@@ -284,6 +284,20 @@ static int do_rollout_gp(const mr_env_state& st, int64_t n, const Params& p, con
     }
 }
 
+template <class T>
+static int do_rollout_collect(const mr_env_state& st, int64_t n, const Params& p, const mr_noise* nz, const TimeView& tv,
+                              const mr_rollout_io& io, const CollectView& cv, const mr_step_out* out, cudaStream_t s) {
+    const RolloutView<T> rv = rollout_view<T>(io);
+    const StateView<T> sv = state_view<T>(st);
+    const OutView<T> ov = out_view<T>(out, n);
+    const NoiseView nv = noise_view(nz, n);
+    switch (nz ? nz->mode : MR_NOISE_NONE) {
+        case MR_NOISE_TABLE: return launch_rollout_collect<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, cv, s);
+        case MR_NOISE_PHILOX: return launch_rollout_collect<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, cv, s);
+        default: return launch_rollout_collect<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, cv, s);
+    }
+}
+
 // the checks of mr_env_rollout that do not depend on the action source
 static int check_rollout(const char* fn, const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
                          const mr_noise* nz, const mr_rollout_io* io, const mr_step_out* out) {
@@ -623,4 +637,43 @@ extern "C" int mr_env_rollout_gp_heading(const mr_env_state* st, int64_t n, int3
     cudaStream_t s = (cudaStream_t)stream;
     return dtype == MR_F64 ? mr::do_rollout_gp<double>(*st, n, pp, nz, tv, *io, gh, out, s)
                            : mr::do_rollout_gp<float>(*st, n, pp, nz, tv, *io, gh, out, s);
+}
+
+extern "C" int mr_env_rollout_ddpg_collect(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                                           const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
+                                           const mr_ddpg_collect* c, const mr_step_out* out, void* stream) {
+    mr::NvtxRange nvtx_range("mr_env_rollout_ddpg_collect");
+    using mr::fail;
+    const char* fn = "mr_env_rollout_ddpg_collect";
+    int rc = mr::check_rollout(fn, st, n, dtype, p, nz, io, out);
+    if (rc) return rc;
+    if (io->action_source != MR_ACTIONS_ACTOR)
+        return fail(MR_ERR_ARG, "%s: io->action_source must be MR_ACTIONS_ACTOR (%d), got %d", fn, MR_ACTIONS_ACTOR, io->action_source);
+    if (!io->actor) return fail(MR_ERR_ARG, "%s: null actor", fn);
+    if (!c) return fail(MR_ERR_ARG, "%s: null collect struct", fn);
+    if (!c->ou_state) return fail(MR_ERR_ARG, "%s: null ou_state", fn);
+    const mr_replay& rb = c->ring;
+    if (!rb.s || !rb.a || !rb.r || !rb.d || !rb.s2) return fail(MR_ERR_ARG, "%s: null replay ring array", fn);
+    if (!out || !out->obs) return fail(MR_ERR_ARG, "%s: the observation rows out->obs (the first policy input) are required", fn);
+    if (rb.capacity <= 0) return fail(MR_ERR_ARG, "%s: ring capacity must be positive", fn);
+    if (c->head < 0 || c->head >= rb.capacity) return fail(MR_ERR_ARG, "%s: need 0 <= head < capacity", fn);
+    if (n > rb.capacity) return fail(MR_ERR_ARG, "%s: more envs than the ring holds (n > capacity)", fn);
+    for (double v : {c->ou_theta, c->ou_mu, c->ou_sigma, c->ou_dt})
+        if (!std::isfinite(v)) return fail(MR_ERR_ARG, "%s: ou_theta, ou_mu, ou_sigma and ou_dt must be finite", fn);
+    if (!tt || !tt->t || tt->len < 2) return fail(MR_ERR_ARG, "%s: time table missing", fn);
+    if (st->a0) return fail(MR_ERR_UNSUPPORTED, "%s: the collector does not take per-env parameter rows", fn);
+    if (mr::g_actor_path == 1) return fail(MR_ERR_UNSUPPORTED, "%s: the CUDA-core actor path (mr_set_actor_path(1)) has no collector", fn);
+    if (n == 0 || io->k_steps == 0) return MR_OK;
+    const mr::Params pp = mr::to_params(*p, nz);
+    const mr::TimeView tv{tt->t, tt->len};
+    mr::CollectView cv;
+    cv.ou = c->ou_state;
+    mr::philox_make_keys(c->ou_seed, cv.keys);
+    cv.theta = c->ou_theta; cv.mu = c->ou_mu; cv.sd = c->ou_sigma * sqrt(c->ou_dt); cv.dt = c->ou_dt;
+    cv.counter = c->ou_counter; cv.env_base = c->ou_env_base;
+    cv.s = rb.s; cv.a = rb.a; cv.r = rb.r; cv.d = rb.d; cv.s2 = rb.s2;
+    cv.capacity = rb.capacity; cv.head = c->head;
+    cudaStream_t s = (cudaStream_t)stream;
+    return dtype == MR_F64 ? mr::do_rollout_collect<double>(*st, n, pp, nz, tv, *io, cv, out, s)
+                           : mr::do_rollout_collect<float>(*st, n, pp, nz, tv, *io, cv, out, s);
 }

@@ -259,4 +259,17 @@ template <class T, int MODE>
 int launch_rollout_gp(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
                       const TimeView& tv, const Params& p, int64_t n, const GpHeadingView& gh, cudaStream_t s);
 
+// DDPG experience collection in the fused rollout (mr_ddpg_collect): the OU process (mr_ou.cuh) and the replay ring.
+struct CollectView {
+    double* ou;                     // [n][2] OU state, in/out
+    PhiloxKeys keys;                // of the OU seed
+    double theta, mu, sd, dt;       // sd = sigma sqrt(dt), as ou_noise_kernel forms it
+    uint64_t counter, env_base;     // step k draws OU sample counter + k of env env_base + i
+    float *s, *a, *r, *d, *s2;      // ring rows [capacity][5] / [capacity][2] / [capacity] / [capacity] / [capacity][5]
+    int64_t capacity, head;         // transition (k, i) goes to slot (head + k n + i) % capacity
+};
+template <class T, int MODE>
+int launch_rollout_collect(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
+                           const TimeView& tv, const Params& p, int64_t n, const CollectView& cv, cudaStream_t s);
+
 }  // namespace mr

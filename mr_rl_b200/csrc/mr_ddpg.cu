@@ -15,6 +15,7 @@
 
 #include "mr_actor.cuh"
 #include "mr_common.cuh"
+#include "mr_ou.cuh"
 
 namespace mr {
 
@@ -546,17 +547,13 @@ __global__ void ou_noise_kernel(double* __restrict__ x, T* __restrict__ actions,
                                 double theta, double mu, double sigma, double dt, PhiloxKeys keys, uint64_t counter, uint64_t env_base) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const uint64_t env = env_base + (uint64_t)i;
-    uint32_t o0, o1, o2, o3;
-    philox4x32_10(3u << 28, (uint32_t)counter, (uint32_t)env, ((uint32_t)(env >> 32) & 0xFFFFu) | ((uint32_t)(counter >> 32) << 16),
-                  keys.rk, o0, o1, o2, o3);
     float z0, z1;
-    box_muller(o0, o1, z0, z1);
+    ou_normals(keys, counter, env_base + (uint64_t)i, z0, z1);
     double x0 = x[2 * i], x1 = x[2 * i + 1];
     if (reset_mask && reset_mask[i]) { x0 = 0.0; x1 = 0.0; }
     const double sd = sigma * sqrt(dt);
-    x0 = x0 + theta * (mu - x0) * dt + sd * (double)z0;
-    x1 = x1 + theta * (mu - x1) * dt + sd * (double)z1;
+    x0 = ou_update(x0, z0, theta, mu, sd, dt);
+    x1 = ou_update(x1, z1, theta, mu, sd, dt);
     x[2 * i] = x0; x[2 * i + 1] = x1;
     actions[2 * i] = (T)((double)actions[2 * i] + x0);
     actions[2 * i + 1] = (T)((double)actions[2 * i + 1] + x1);

@@ -254,8 +254,35 @@ class DDPGLearner:
         return _unpack(self.critic_target if target else self.critic, CRITIC_ORDER, CRITIC_SHAPES)
 
 
+def collect(env, learner, actor_noise, replay, k_steps, **rollout_kw):
+    """K iterations of train()'s acting loop in ONE launch: per step, every env acts with mu(s) + the next OU sample, steps,
+    and its transition (s, a, r, done, s2) enters the replay ring.  Uses the online actor ``learner.actor`` as it is at
+    launch time, the noise's state / call count / seed / env base and the ring's head.  Afterwards ``replay.head`` /
+    ``replay.count`` and ``actor_noise.calls`` have advanced exactly as K ``add`` / ``add_to`` calls advance them; the stream
+    is not synchronised.  On the 3xTF32 actor path (``_lib.set_actor_path("tf32")``) the ring, the noise state and the env
+    equal K rounds of predict -> add_to -> step -> add bit for bit; the default 3xFP16 path agrees to ~1e-4 of the action
+    range.  ``rollout_kw`` go to ``env.rollout`` (recording rows, statistics, reset_init), whose result is returned."""
+    k = int(k_steps)
+    n = env.num_envs
+    if k < 1:
+        raise ValueError("k_steps must be at least 1")
+    if n > replay.buffer_size:
+        raise ValueError(f"{n} envs add more transitions per step than the replay buffer holds ({replay.buffer_size})")
+    if actor_noise.x_prev.shape[0] < n:
+        raise ValueError(f"the OU noise has {actor_noise.x_prev.shape[0]} processes for {n} envs")
+    if tuple(learner.action_bound) != (env.params.action_high[0], env.params.action_high[1]):
+        raise ValueError("learner.action_bound must equal the env's action_space.high (the in-kernel actor scales by it)")
+    c = L.DDPGCollect(actor_noise.x_prev.data_ptr(), actor_noise.theta, actor_noise.mu, actor_noise.sigma, actor_noise.dt,
+                      actor_noise.seed & (2**64 - 1), actor_noise.calls, actor_noise.env_base, replay._c, replay.head)
+    res = env.rollout(policy=learner.actor, k_steps=k, ddpg_collect=c, **rollout_kw)
+    replay.head = (replay.head + k * n) % replay.buffer_size
+    replay.count = min(replay.count + k * n, replay.buffer_size)
+    actor_noise.calls += k
+    return res
+
+
 def train(env, learner, actor_noise, buffer_size=10000, min_batch=64, steps=1000, updates_per_step=1, replay=None,
-          noise_var=1, a0=1, log_every=0, stale_state_warmup=False):
+          noise_var=1, a0=1, log_every=0, stale_state_warmup=False, collect_steps=None):
     """train() (:233-323) for a vectorised env: every iteration all N envs act with mu(s) + OU noise, the N transitions
     enter the ring, and once it holds ``min_batch`` transitions the learner takes ``updates_per_step`` updates.  ``env``
     is a VecMREnv built with auto_reset=True (an env that ends starts its next episode inside the same launch, the
@@ -264,8 +291,18 @@ def train(env, learner, actor_noise, buffer_size=10000, min_batch=64, steps=1000
     ``stale_state_warmup=True`` reproduces the scalar loop's warm-up quirk: while the buffer holds fewer than
     ``min_batch`` transitions the loop ``continue``s before ``state = next_state`` (:281-284), so the policy keeps seeing —
     and the buffer keeps storing as ``s`` — the observation of the last reset, while the env itself moves on.  With
-    N >= min_batch envs the buffer is full after the first iteration and the flag changes nothing."""
+    N >= min_batch envs the buffer is full after the first iteration and the flag changes nothing.
+    ``collect_steps=K`` fuses the acting: an iteration is one ``collect`` of K env steps (the last one shorter if K does
+    not divide ``steps``), then K * ``updates_per_step`` updates once the ring holds ``min_batch`` transitions — the same
+    ratio of updates to env steps, with a policy up to K steps stale.  The log then has one row per launch: the mean
+    reward over its transitions (from the env's statistics vector, which these launches accumulate) and the loss and
+    mean Q of its last update.  ``collect_steps=1`` on the 3xTF32 actor path reproduces the default loop bit for bit."""
     n = env.num_envs
+    if collect_steps is not None:
+        if stale_state_warmup:
+            raise ValueError("stale_state_warmup reproduces the per-step loop; it cannot be combined with collect_steps")
+        return _train_collect(env, learner, actor_noise, buffer_size, min_batch, steps, updates_per_step, replay,
+                              noise_var, a0, log_every, int(collect_steps))
     replay = replay if replay is not None else ReplayBuffer(buffer_size, 0, device=env.device)
     obs_rows = env._obs
     env.reset(noise_var=noise_var, a0=a0)
@@ -290,4 +327,33 @@ def train(env, learner, actor_noise, buffer_size=10000, min_batch=64, steps=1000
         if log_every and (it + 1) % log_every == 0:
             row = log[it].cpu().numpy()
             print(f"iter {it + 1}/{steps}: mean reward {row[0]:.3f} critic loss {row[1]:.4g} mean Q {row[2]:.4g}")
+    return log.cpu().numpy()
+
+
+def _train_collect(env, learner, actor_noise, buffer_size, min_batch, steps, updates_per_step, replay, noise_var, a0,
+                   log_every, k):
+    n = env.num_envs
+    if k < 1:
+        raise ValueError("collect_steps must be at least 1")
+    replay = replay if replay is not None else ReplayBuffer(buffer_size, 0, device=env.device)
+    if n > replay.buffer_size:
+        raise ValueError(f"{n} envs add more transitions per step than the replay buffer holds ({replay.buffer_size})")
+    env.reset(noise_var=noise_var, a0=a0)
+    launches = (steps + k - 1) // k
+    log = torch.zeros(launches, 3, dtype=torch.float64, device=env.device)
+    rew_sum = env.stats[L.STAT_NAMES.index("sum_reward")]
+    done = 0
+    for it in range(launches):
+        kk = min(k, steps - done)
+        before = rew_sum.clone()
+        collect(env, learner, actor_noise, replay, kk)
+        log[it, 0] = (rew_sum - before) / (kk * n)
+        if replay.size() >= min_batch:
+            for _ in range(kk * updates_per_step):
+                info = learner.update(replay, min_batch)
+            log[it, 1:] = info.double()
+        done += kk
+        if log_every and (it + 1) % log_every == 0:
+            row = log[it].cpu().numpy()
+            print(f"launch {it + 1}/{launches} ({done} steps): mean reward {row[0]:.3f} critic loss {row[1]:.4g} mean Q {row[2]:.4g}")
     return log.cpu().numpy()

@@ -524,7 +524,7 @@ class VecMREnv:
 
     # ---- fused K-step rollout: utils.run_sim (utils.py:43-61) / the DDPG acting loop --------------
     def rollout(self, actions=None, k_steps=None, policy=None, record=False, record_state_prime=False,
-                record_done=False, accumulate_stats=True, record_episodes=False, reset_init=None):
+                record_done=False, accumulate_stats=True, record_episodes=False, reset_init=None, ddpg_collect=None):
         """K env steps in ONE launch with the state held in registers.
 
         actions : [K, N, 2] per-env actions, or [K, 2] / [K, >=2] one action row for every env
@@ -540,12 +540,14 @@ class VecMREnv:
                   the reference's pickle layout.  Episode ordinals continue across launches (``self._episode_counter``).
         reset_init : [E, N, 2] start positions for the auto resets (episode e of env i restarts at reset_init[(e-1) % E, i])
                   instead of sampling init_space.
+        ddpg_collect : with an actor ``policy``, the ``_lib.DDPGCollect`` of ``ddpg.collect``: the launch also adds OU
+                  noise to the actions and writes every transition into the replay ring (mr_env_rollout_ddpg_collect).
         Returns dict(obs, rew, done[, xy [K,2,N], state_prime [K,2,N], done_traj [K,N]]).
         """
         if torch.cuda.current_device() != self._dev_index:
             with torch.cuda.device(self.device):
                 return self.rollout(actions, k_steps, policy, record, record_state_prime, record_done, accumulate_stats,
-                                    record_episodes, reset_init)
+                                    record_episodes, reset_init, ddpg_collect)
         n = self.num_envs
         io = L.RolloutIO()
         keep = []
@@ -584,6 +586,8 @@ class VecMREnv:
             keep.extend(tensors)
         else:
             raise ValueError("give actions or policy")
+        if ddpg_collect is not None and io.action_source != L.ACTIONS_ACTOR:
+            raise ValueError("ddpg_collect needs an actor policy")
         io.k_steps = k
         res = {}
         if record_episodes:
@@ -626,6 +630,11 @@ class VecMREnv:
                                                     C.byref(self._c_tt), C.byref(io), C.byref(gp_pol), C.byref(self._c_out),
                                                     self._stream())
             L.check(rc, "mr_env_rollout_gp_heading")
+        elif ddpg_collect is not None:
+            rc = self.lib.mr_env_rollout_ddpg_collect(C.byref(self._c_state), n, self._dt, C.byref(self.params), C.byref(nz),
+                                                      C.byref(self._c_tt), C.byref(io), C.byref(ddpg_collect),
+                                                      C.byref(self._c_out), self._stream())
+            L.check(rc, "mr_env_rollout_ddpg_collect")
         else:
             rc = self.lib.mr_env_rollout(C.byref(self._c_state), n, self._dt, C.byref(self.params), C.byref(nz),
                                          C.byref(self._c_tt), C.byref(io), C.byref(self._c_out), self._stream())
