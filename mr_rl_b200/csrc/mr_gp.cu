@@ -55,8 +55,9 @@ gp_kq_mean_kernel(const double* __restrict__ q, int64_t n_q, const double* __res
 
 // exp(x) for x <= 0 with a 64-entry table of 2^(j/64) in shared memory and a degree-5 polynomial:
 // x = (64 m + j) ln2/64 + r, |r| <= ln2/128, exp(x) = 2^m * T[j] * (1 + r + ... + r^5/120) (truncation
-// 3.5e-17).  ~14 fp64 instructions instead of the ~25 of the library exp; ~2 ulp.  Results below
-// 2^-1021 flush to 0 (such kernel values cannot influence a sum whose other terms are O(1e-300) larger).
+// 3.5e-17).  ~14 fp64 instructions instead of the ~25 of the library exp; at most 2 ulp (tested down to
+// x = -745).  Results below 2^-1021 flush to 0 (such kernel values cannot influence a sum whose other terms
+// are O(1e-300) larger).
 __device__ __forceinline__ void exp_table_init(double* T) {
     if (threadIdx.x < 64) T[threadIdx.x] = exp2((double)threadIdx.x / 64.0);
 }
@@ -64,8 +65,9 @@ __device__ __forceinline__ double exp_neg_tab(double x, const double* __restrict
     const double t = x * 92.33248261689366;                      // 64 / ln 2
     const int n = __double2int_rn(t);
     const double nd = (double)n;
-    double r = fma(-nd, 0x1.62e42fefa0000p-7, x);                // ln2/64, high 36 bits (n * hi is exact)
-    r = fma(-nd, 0x1.cf78000000000p-46, r);                      // ... and the remainder
+    double r = fma(-nd, 0x1.62e42fefa0000p-7, x);                // ln2/64 = hi + lo: hi its leading 36 bits,
+    r = fma(-nd, 0x1.cf79abc9e3b3ap-46, r);                      // lo the correctly rounded rest (a shorter lo
+                                                                 // biases every result low by ~3.3e-17 |x|)
     double p = fma(r, 1.0 / 120.0, 1.0 / 24.0);
     p = fma(p, r, 1.0 / 6.0);
     p = fma(p, r, 0.5);
@@ -73,8 +75,11 @@ __device__ __forceinline__ double exp_neg_tab(double x, const double* __restrict
     p = fma(p, r, 1.0);
     const int m = n >> 6;                                        // floor division: j = n & 63 in [0, 63]
     const double v = T[n & 63] * p;                              // in [1, 2.04)
-    if (m < -1021) return 0.0;
-    return __longlong_as_double(__double_as_longlong(v) + ((long long)m << 52));
+    const double y = __longlong_as_double(__double_as_longlong(v) + ((long long)m << 52));
+    // flush when m < -1021, i.e. rint(t) <= -65345, i.e. t < -65344.5 (the tie rounds to the even -65344).  Tested on t
+    // rather than m: a NaN x converts to n = INT_MIN like -inf, but fails this comparison and stays NaN through r, p
+    // and v (INT_MIN >> 6 << 52 adds 0), so a NaN query gives a NaN posterior instead of the prior.
+    return t < -65344.5 ? 0.0 : y;
 }
 
 // ---- kernel 1 (staged): training points and alpha live in shared memory ---------------------
@@ -627,8 +632,9 @@ int mr_gp_predict(const mr_gp_model* gp, const double* q, int64_t n_q, double* m
     if (n_q == 0) return MR_OK;
     if (!q || !mean) return fail(MR_ERR_ARG, "mr_gp_predict: null q/mean");
     if (gp->dim != 1 && gp->dim != 2) return fail(MR_ERR_UNSUPPORTED, "mr_gp_predict: dim must be 1 or 2");
-    if (gp->n_pad % MR_GP_PAD != 0 || gp->n_train > gp->n_pad || gp->n_train <= 0)
-        return fail(MR_ERR_ARG, "mr_gp_predict: n_pad must be a multiple of %d and >= n_train", MR_GP_PAD);
+    if (gp->n_pad <= 0 || gp->n_pad % MR_GP_PAD != 0)
+        return fail(MR_ERR_ARG, "mr_gp_predict: n_pad must be a positive multiple of %d", MR_GP_PAD);
+    if (gp->n_train > gp->n_pad || gp->n_train <= 0) return fail(MR_ERR_ARG, "mr_gp_predict: need 1 <= n_train <= n_pad");
     if (!(gp->length_scale > 0)) return fail(MR_ERR_ARG, "mr_gp_predict: bad length_scale");
     cudaStream_t s = (cudaStream_t)stream;
     if (!std) {
@@ -664,8 +670,8 @@ int mr_gp_predict(const mr_gp_model* gp, const double* q, int64_t n_q, double* m
     if (!workspace || workspace_bytes < mr_gp_workspace_bytes(gp, n_q, 1))
         return fail(MR_ERR_ARG, "mr_gp_predict: workspace too small (%lld < %lld)", (long long)workspace_bytes,
                     (long long)mr_gp_workspace_bytes(gp, n_q, 1));
-    if (((uintptr_t)workspace & 15u) || ((uintptr_t)gp->linv & 15u))
-        return fail(MR_ERR_ARG, "mr_gp_predict: workspace / linv must be 16-byte aligned");
+    if ((uintptr_t)workspace & 15u) return fail(MR_ERR_ARG, "mr_gp_predict: workspace must be 16-byte aligned");
+    if ((uintptr_t)gp->linv & 15u) return fail(MR_ERR_ARG, "mr_gp_predict: linv must be 16-byte aligned");
     const int64_t chunk_cap = round_up(n_q < kGpChunk ? n_q : kGpChunk, GP_BM);
     double* kq = (double*)workspace;
     double* ssq = kq + chunk_cap * gp->n_pad;
