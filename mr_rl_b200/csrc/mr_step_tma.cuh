@@ -212,10 +212,13 @@ template <class T, int MODE> struct TmaMinCtas {
 // obs (x, y) pair, the goal pair, the state_prime pair, the tile's 16 / 24 noise-table rows) instead of one 1-D bulk copy
 // per row: 8-9 copy instructions per tile instead of 19-20 (table mode 10 instead of 36), all issued by one thread that
 // also integrates an env, i.e. by the warp every other warp of the CTA waits for at the tile's two barriers.
-template <class T, int MODE, bool MISM, bool TMAP>
+// STD: the launch has the standard outputs — actions and output rows in the storage type, obs with its goal rows, rew and
+// done, no state_prime, auto reset on — so the per-tile tests of those options fold away at compile time (tensor maps only).
+template <class T, int MODE, bool MISM, bool TMAP, bool STD = false>
 __global__ void __launch_bounds__(TileOf<T>::value, TmaMinCtas<T, MODE>::value)
 env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> out, NoiseView nv, TimeView tv,
                     Params p, int64_t n_tiles, int64_t n_total, const __grid_constant__ StepMaps maps) {
+    static_assert(!STD || TMAP, "the standard-output form moves its rows with tensor maps");
     constexpr int kTile = TileOf<T>::value;
     constexpr int kSI = StagesIn<MODE>::value;
     constexpr int kNR = NoiseRows<MODE, MISM>::value;
@@ -241,8 +244,11 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
     asm volatile("griddepcontrol.wait;" ::: "memory");
 
     constexpr uint32_t kRow = kTile * sizeof(T);
-    const bool act32 = sizeof(T) == 8 && p.act_f32;         // float32 actions with fp64 storage (mr_sim_params.action_f32)
-    const bool out32 = sizeof(T) == 8 && out.f32;           // float32 output rows with fp64 storage (mr_step_out.out_f32)
+    const bool act32 = !STD && sizeof(T) == 8 && p.act_f32;  // float32 actions with fp64 storage (mr_sim_params.action_f32)
+    const bool out32 = !STD && sizeof(T) == 8 && out.f32;    // float32 output rows with fp64 storage (mr_step_out.out_f32)
+    const bool w_obs = STD || out.obs, w_goal = STD || out.goal, w_rew = STD || out.rew, w_done = STD || out.done;
+    const bool w_sp = !STD && out.sp;
+    const bool auto_reset = STD || p.auto_reset;
     const uint32_t act_bytes = act32 ? kTile * 8u : 2u * kRow;
     const uint32_t kInBytes = 5 * kRow + act_bytes + kTile * 4;
     const uint64_t off = step_offset(nv);                   // env-step index of this launch (after griddepcontrol.wait)
@@ -259,9 +265,17 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
     constexpr int kWarps = MR_ISSUE_WARPS;                  // 1: a single issuing thread
     const int warp = tid >> 5;
     const bool elect = (tid & 31) == 0 && warp < kWarps;
+    // Copy plumbing hoisted out of the tile loop: a CTA's tiles start kTile * gridDim.x envs apart and n < 2^31, so the
+    // loop advances one unsigned 32-bit env index (a few tiles past the end it still compares correctly) that is also the
+    // TMA coordinate, and every row address is a base fixed before the loop plus that index.
+    const uint32_t env_stride = (uint32_t)stride * kTile;
+    const uint32_t n_full = (uint32_t)(n_tiles * kTile);   // envs covered by whole tiles
+    const char* const act_base = (const char*)actions;
+    const uint32_t act_el = act32 ? 8u : 2u * (uint32_t)sizeof(T);   // action bytes per env
+    int32_t* const ctr_row = st.counter;
+    T* const d_row = w_obs ? out.obs + 4 * out.stride : nullptr;
     // cbase (table mode): the noise cursor of the tile's first env = first table row to stage
-    auto issue_loads = [&](int s, int64_t tile, int32_t cbase) {     // called by the elected lane of every warp
-        const int64_t i0 = tile * kTile;
+    auto issue_loads = [&](int s, uint32_t i0, int32_t cbase) {       // called by the elected lane of every warp
         uint64_t* bar = &sm.full[s];
         TileIn<T, kTile>& b = sm.in[s];
         if constexpr (kTable) {
@@ -290,46 +304,43 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
             if (warp == 3 % kWarps) bulk_load(b.fy, st.fy + i0, kRow, bar);
             if (warp == 4 % kWarps) bulk_load(b.h, st.h + i0, kRow, bar);
         }
-        if (warp == 5 % kWarps)
-            bulk_load(b.act, act32 ? (const void*)(reinterpret_cast<const float*>(actions) + 2 * i0) : (const void*)(actions + 2 * i0),
-                      act_bytes, bar);
-        if (warp == 6 % kWarps) bulk_load(b.counter, st.counter + i0, kTile * 4, bar);
+        if (warp == 5 % kWarps) bulk_load(b.act, act_base + (int64_t)i0 * act_el, act_bytes, bar);
+        if (warp == 6 % kWarps) bulk_load(b.counter, ctr_row + i0, kTile * 4, bar);
     };
     // this launch changes a tile's cursors only when it processes the tile, so the elected thread may read the first
     // cursor of a tile it will load later with a plain load, one issue ahead (its latency hides behind a tile)
-    auto tile_cursor = [&](int64_t tile) -> int32_t {
-        if constexpr (kTable) { if (tile < n_tiles) return st.cursor[tile * kTile]; }
+    auto tile_cursor = [&](uint32_t i0) -> int32_t {
+        if constexpr (kTable) { if (i0 < n_full) return st.cursor[i0]; }
         return 0;
     };
 
     int32_t cb_next = 0;
+    const uint32_t first_i0 = (uint32_t)first * kTile;
     if (elect) {
         for (int s = 0; s < kSI; ++s) {
-            const int64_t tile = first + (int64_t)s * stride;
-            if (tile < n_tiles) issue_loads(s, tile, tile_cursor(tile));
+            const uint32_t i0 = first_i0 + s * env_stride;
+            if (i0 < n_full) issue_loads(s, i0, tile_cursor(i0));
         }
-        cb_next = tile_cursor(first + (int64_t)kSI * stride);
+        cb_next = tile_cursor(first_i0 + kSI * env_stride);
     }
 
     constexpr bool kPrefetch = MR_RNG_PREFETCH && MODE == MR_NOISE_PHILOX && !MISM;
-    auto predraw = [&](int64_t tile) {                      // this thread's normals for `tile`, parked in shared memory
+    auto predraw = [&](uint32_t i0) {                       // this thread's normals for tile i0, parked in shared memory
         if constexpr (kPrefetch) {
             PhiloxNoise nzp;
-            nzp.seek(nv.env_base + (uint64_t)(tile * kTile + tid), off);
+            nzp.seek(nv.env_base + (uint64_t)(i0 + tid), off);
             float z8[8];
             nzp.draw8(p, z8);
             sm.zpre[tid] = make_float4(z8[0], z8[1], z8[2], z8[3]);
             sm.zpre[kTile + tid] = make_float4(z8[4], z8[5], z8[6], z8[7]);
         }
     };
-    if (first < n_tiles) predraw(first);
+    if (first_i0 < n_full) predraw(first_i0);
 
-    int it = 0;
-    for (int64_t tile = first; tile < n_tiles; tile += stride, ++it) {
-        const int s = it % kSI;
-        const uint32_t parity = (uint32_t)(it / kSI) & 1u;
-        const int so = it % kSO;
-        const int64_t i0 = tile * kTile;
+    int s = 0, so = 0;                                      // input / output stage of this tile
+    uint32_t parity = 0;                                    // phase of full[s] this tile waits for
+    for (uint32_t i0 = first_i0; i0 < n_full; i0 += env_stride) {
+        const uint32_t nxt = i0 + kSI * env_stride;         // the tile whose loads re-fill in[s]
 
         mbar_wait(&sm.full[s], parity);
         Env e;
@@ -345,10 +356,7 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
             if (elect) bulk_wait_read<kStagesOut - 1>();    // out[so] (used kStagesOut tiles ago) has been read out
             __syncthreads();                                // [A] in[s] fully consumed, out[so] free
             if constexpr (!kTable) {
-                if (elect) {
-                    const int64_t nxt = tile + (int64_t)kSI * stride;
-                    if (nxt < n_tiles) issue_loads(s, nxt, 0);
-                }
+                if (elect && nxt < n_full) issue_loads(s, nxt, 0);
             }
         }
 
@@ -369,7 +377,7 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
         } else if constexpr (kPrefetch) {
             const float4 za = sm.zpre[tid], zb = sm.zpre[kTile + tid];
             const float z8[8] = {za.x, za.y, za.z, za.w, zb.x, zb.y, zb.z, zb.w};
-            if (tile + stride < n_tiles) predraw(tile + stride);      // independent of everything below
+            if (i0 + env_stride < n_full) predraw(i0 + env_stride);   // independent of everything below
             PhiloxNoise nz;                                     // only the rare multi-attempt path draws from it
             nz.seek(nv.env_base + (uint64_t)(i0 + tid), off);
             nz.blk += 2;
@@ -380,7 +388,7 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
         }
         const Observation o = observe(e, p);
         double d_out = o.d, il_next = tb2 - tb;
-        if (p.auto_reset && o.done) {                       // reported obs = first obs of the new episode
+        if (auto_reset && o.done) {                         // reported obs = first obs of the new episode
             int ov = 0;
             auto_reset_env<MODE, MISM>(e, nv, n_total, i0 + tid, cur, off, p, ov);
             if (ov) e.status |= kNoiseOverflow;
@@ -398,10 +406,10 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
             // rew <- x | y,  d <- d | rew,  spx <- spx | spy
             float* fxy = reinterpret_cast<float*>(bo.rew); fxy[tid] = (float)e.x; fxy[kTile + tid] = (float)e.y;
             float* fdr = reinterpret_cast<float*>(bo.d); fdr[tid] = (float)d_out; fdr[kTile + tid] = (float)o.rew;
-            if (out.sp) { float* fsp = reinterpret_cast<float*>(bo.spx); fsp[tid] = (float)e.spx; fsp[kTile + tid] = (float)e.spy; }
+            if (w_sp) { float* fsp = reinterpret_cast<float*>(bo.spx); fsp[tid] = (float)e.spx; fsp[kTile + tid] = (float)e.spy; }
         } else {
             bo.d[tid] = (T)d_out; bo.rew[tid] = (T)o.rew;
-            if (out.sp) { bo.spx[tid] = (T)e.spx; bo.spy[tid] = (T)e.spy; }
+            if (w_sp) { bo.spx[tid] = (T)e.spx; bo.spy[tid] = (T)e.spy; }
         }
         if constexpr (kTable) sm.nout[so].cursor[tid] = cur;
         if (e.status) st.status[i0 + tid] |= (uint8_t)e.status;   // rare: sticky flags, plain store
@@ -409,36 +417,34 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
         __syncthreads();                                    // [B] tile results complete in out[so]
         if (elect) {
             if constexpr (kOneBar) {                        // in[s] was copied to registers before [B] by every thread
-                const int64_t nxt = tile + (int64_t)kSI * stride;
-                if (nxt < n_tiles) issue_loads(s, nxt, 0);
+                if (nxt < n_full) issue_loads(s, nxt, 0);
             }
             if constexpr (kTable) {                         // the stage's noise rows are free only now
-                const int64_t nxt = tile + (int64_t)kSI * stride;
-                if (nxt < n_tiles) issue_loads(s, nxt, cb_next);
-                cb_next = tile_cursor(nxt + stride);
+                if (nxt < n_full) issue_loads(s, nxt, cb_next);
+                cb_next = tile_cursor(nxt + env_stride);
                 bulk_store(st.cursor + i0, sm.nout[so].cursor, kTile * 4);
             }
             if constexpr (TMAP) {
                 tensor_store_2d(&maps.state, (int32_t)i0, 0, bo.x);                              // x, y, fx, fy, h
-                bulk_store(st.counter + i0, bo.counter, kTile * 4);
+                bulk_store(ctr_row + i0, bo.counter, kTile * 4);
                 if (out32) {
                     constexpr uint32_t kRow32 = kTile * 4;
                     const float* fdr = reinterpret_cast<const float*>(bo.d);
-                    if (out.obs) {
+                    if (w_obs) {
                         tensor_store_2d(&maps.obs, (int32_t)i0, 0, bo.rew);                      // float x | y
-                        if (out.goal) tensor_store_2d(&maps.obs, (int32_t)i0, 2, sm.zero);
+                        if (w_goal) tensor_store_2d(&maps.obs, (int32_t)i0, 2, sm.zero);
                         bulk_store(reinterpret_cast<float*>(out.obs) + 4 * out.stride + i0, fdr, kRow32);
                     }
-                    if (out.rew) bulk_store(reinterpret_cast<float*>(out.rew) + i0, fdr + kTile, kRow32);
-                    if (out.sp) tensor_store_2d(&maps.sp, (int32_t)i0, 0, bo.spx);               // float spx | spy
+                    if (w_rew) bulk_store(reinterpret_cast<float*>(out.rew) + i0, fdr + kTile, kRow32);
+                    if (w_sp) tensor_store_2d(&maps.sp, (int32_t)i0, 0, bo.spx);                 // float spx | spy
                 } else {
-                    if (out.obs) {
+                    if (w_obs) {
                         tensor_store_2d(&maps.obs, (int32_t)i0, 0, bo.x);                        // obs rows x, y
-                        if (out.goal) tensor_store_2d(&maps.obs, (int32_t)i0, 2, sm.zero);       // goal = (0,0), MR_env.py:57
-                        bulk_store(out.obs + 4 * out.stride + i0, bo.d, kRow);
+                        if (w_goal) tensor_store_2d(&maps.obs, (int32_t)i0, 2, sm.zero);         // goal = (0,0), MR_env.py:57
+                        bulk_store(d_row + i0, bo.d, kRow);
                     }
-                    if (out.rew) bulk_store(out.rew + i0, bo.rew, kRow);
-                    if (out.sp) tensor_store_2d(&maps.sp, (int32_t)i0, 0, bo.spx);
+                    if (w_rew) bulk_store(out.rew + i0, bo.rew, kRow);
+                    if (w_sp) tensor_store_2d(&maps.sp, (int32_t)i0, 0, bo.spx);
                 }
             } else {
             if (warp == 0 % kWarps) bulk_store(st.x + i0, bo.x, kRow);
@@ -482,10 +488,12 @@ env_step_tma_kernel(StateView<T> st, const T* __restrict__ actions, OutView<T> o
                 }
             }
             }
-            if (out.done && warp == 12 % kWarps) bulk_store(out.done + i0, bo.done, kTile);
+            if (w_done && warp == 12 % kWarps) bulk_store(out.done + i0, bo.done, kTile);
             bulk_commit();                                  // bulk groups are per thread: every issuing lane commits
             if constexpr (kOneBar) bulk_wait_read<1>();     // tile it-1's stores have been read out: frees out[(it + 2) % 3]
         }
+        if (++s == kSI) { s = 0; parity ^= 1u; }
+        if (++so == kSO) so = 0;
     }
     if (elect) bulk_wait_read<0>();                         // smem must outlive the last bulk stores
 }
