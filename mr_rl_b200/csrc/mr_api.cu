@@ -258,43 +258,16 @@ static RolloutView<T> rollout_view(const mr_rollout_io& io) {
 
 template <class T>
 static int do_rollout(const mr_env_state& st, int64_t n, const Params& p, const mr_noise* nz, const TimeView& tv,
-                      const mr_rollout_io& io, const mr_step_out* out, cudaStream_t s) {
+                      const mr_rollout_io& io, const GpHeadingView* gh, const CollectView* cv, const mr_step_out* out,
+                      cudaStream_t s) {
     const RolloutView<T> rv = rollout_view<T>(io);
     const StateView<T> sv = state_view<T>(st);
     const OutView<T> ov = out_view<T>(out, n);
     const NoiseView nv = noise_view(nz, n);
     switch (nz ? nz->mode : MR_NOISE_NONE) {
-        case MR_NOISE_TABLE: return launch_rollout<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, s);
-        case MR_NOISE_PHILOX: return launch_rollout<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, s);
-        default: return launch_rollout<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, s);
-    }
-}
-
-template <class T>
-static int do_rollout_gp(const mr_env_state& st, int64_t n, const Params& p, const mr_noise* nz, const TimeView& tv,
-                         const mr_rollout_io& io, const GpHeadingView& gh, const mr_step_out* out, cudaStream_t s) {
-    const RolloutView<T> rv = rollout_view<T>(io);
-    const StateView<T> sv = state_view<T>(st);
-    const OutView<T> ov = out_view<T>(out, n);
-    const NoiseView nv = noise_view(nz, n);
-    switch (nz ? nz->mode : MR_NOISE_NONE) {
-        case MR_NOISE_TABLE: return launch_rollout_gp<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, gh, s);
-        case MR_NOISE_PHILOX: return launch_rollout_gp<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, gh, s);
-        default: return launch_rollout_gp<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, gh, s);
-    }
-}
-
-template <class T>
-static int do_rollout_collect(const mr_env_state& st, int64_t n, const Params& p, const mr_noise* nz, const TimeView& tv,
-                              const mr_rollout_io& io, const CollectView& cv, const mr_step_out* out, cudaStream_t s) {
-    const RolloutView<T> rv = rollout_view<T>(io);
-    const StateView<T> sv = state_view<T>(st);
-    const OutView<T> ov = out_view<T>(out, n);
-    const NoiseView nv = noise_view(nz, n);
-    switch (nz ? nz->mode : MR_NOISE_NONE) {
-        case MR_NOISE_TABLE: return launch_rollout_collect<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, cv, s);
-        case MR_NOISE_PHILOX: return launch_rollout_collect<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, cv, s);
-        default: return launch_rollout_collect<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, cv, s);
+        case MR_NOISE_TABLE: return launch_rollout<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, gh, cv, s);
+        case MR_NOISE_PHILOX: return launch_rollout<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, gh, cv, s);
+        default: return launch_rollout<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, gh, cv, s);
     }
 }
 
@@ -599,8 +572,8 @@ int mr_env_rollout(const mr_env_state* st, int64_t n, int32_t dtype, const mr_si
     const mr::Params pp = mr::to_params(*p, nz);
     mr::TimeView tv{tt->t, tt->len};
     cudaStream_t s = (cudaStream_t)stream;
-    return dtype == MR_F64 ? mr::do_rollout<double>(*st, n, pp, nz, tv, *io, out, s)
-                           : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, out, s);
+    return dtype == MR_F64 ? mr::do_rollout<double>(*st, n, pp, nz, tv, *io, nullptr, nullptr, out, s)
+                           : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, nullptr, nullptr, out, s);
 }
 
 }  // extern "C"
@@ -635,8 +608,8 @@ extern "C" int mr_env_rollout_gp_heading(const mr_env_state* st, int64_t n, int3
     gh.lo = -3.141592653589793; gh.hi = 3.141592653589793; gh.xatol = 1e-5;
     gh.n_coef = pol->n_coef; gh.maxfun = 500;
     cudaStream_t s = (cudaStream_t)stream;
-    return dtype == MR_F64 ? mr::do_rollout_gp<double>(*st, n, pp, nz, tv, *io, gh, out, s)
-                           : mr::do_rollout_gp<float>(*st, n, pp, nz, tv, *io, gh, out, s);
+    return dtype == MR_F64 ? mr::do_rollout<double>(*st, n, pp, nz, tv, *io, &gh, nullptr, out, s)
+                           : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, &gh, nullptr, out, s);
 }
 
 extern "C" int mr_env_rollout_ddpg_collect(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
@@ -674,6 +647,6 @@ extern "C" int mr_env_rollout_ddpg_collect(const mr_env_state* st, int64_t n, in
     cv.s = rb.s; cv.a = rb.a; cv.r = rb.r; cv.d = rb.d; cv.s2 = rb.s2;
     cv.capacity = rb.capacity; cv.head = c->head;
     cudaStream_t s = (cudaStream_t)stream;
-    return dtype == MR_F64 ? mr::do_rollout_collect<double>(*st, n, pp, nz, tv, *io, cv, out, s)
-                           : mr::do_rollout_collect<float>(*st, n, pp, nz, tv, *io, cv, out, s);
+    return dtype == MR_F64 ? mr::do_rollout<double>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s)
+                           : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s);
 }

@@ -34,6 +34,15 @@ inline int current_device() {
     cudaGetDevice(&dev);
     return dev >= 0 && dev < kMaxDevices ? dev : 0;
 }
+// SMs of device `dev` (an index from current_device()), queried once per device
+inline int sm_count(int dev) {
+    static int cached[kMaxDevices] = {};
+    if (!cached[dev]) {
+        cudaDeviceGetAttribute(&cached[dev], cudaDevAttrMultiProcessorCount, dev);
+        if (cached[dev] <= 0) cached[dev] = 148;
+    }
+    return cached[dev];
+}
 
 // ---- device-side views ---------------------------------------------------------------------
 template <class T>
@@ -240,9 +249,6 @@ struct RolloutView {
     int k_steps;
     int action_source;
 };
-template <class T, int MODE>
-int launch_rollout(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
-                   const TimeView& tv, const Params& p, int64_t n, cudaStream_t s);
 
 // The GP-corrected heading policy of the fused rollout (mr_gp_heading_policy): per env and step k the desired velocity
 // vd = v_ref[k] + gain (p_ref[k] - p), then the heading search of gp_correct_heading_cheb_kernel on [lo, hi].
@@ -255,9 +261,6 @@ struct GpHeadingView {
     double lo, hi, xatol;      // search interval and tolerance, passed at run time as the standalone kernel takes them
     int n_coef, maxfun;
 };
-template <class T, int MODE>
-int launch_rollout_gp(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
-                      const TimeView& tv, const Params& p, int64_t n, const GpHeadingView& gh, cudaStream_t s);
 
 // DDPG experience collection in the fused rollout (mr_ddpg_collect): the OU process (mr_ou.cuh) and the replay ring.
 struct CollectView {
@@ -268,8 +271,11 @@ struct CollectView {
     float *s, *a, *r, *d, *s2;      // ring rows [capacity][5] / [capacity][2] / [capacity] / [capacity] / [capacity][5]
     int64_t capacity, head;         // transition (k, i) goes to slot (head + k n + i) % capacity
 };
+// The fused rollout of every action source.  gh: the GP heading policy, only from mr_env_rollout_gp_heading; cv: the
+// DDPG collector, only from mr_env_rollout_ddpg_collect; both null from mr_env_rollout.
 template <class T, int MODE>
-int launch_rollout_collect(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
-                           const TimeView& tv, const Params& p, int64_t n, const CollectView& cv, cudaStream_t s);
+int launch_rollout(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
+                   const TimeView& tv, const Params& p, int64_t n, const GpHeadingView* gh, const CollectView* cv,
+                   cudaStream_t s);
 
 }  // namespace mr

@@ -661,9 +661,7 @@ int mr_ddpg_update(const mr_ddpg_state* st, const mr_replay* rb, int64_t count, 
     int64_t* idx = (int64_t*)workspace;
     float* slabs = (float*)((char*)workspace + (((int64_t)batch * 8 + 63) / 64) * 64);
     const int tiles = (batch + kTile - 1) / kTile;
-    static int sm_counts[kMaxDevices] = {};
-    if (!sm_counts[dev]) cudaDeviceGetAttribute(&sm_counts[dev], cudaDevAttrMultiProcessorCount, dev);
-    const int sms = sm_counts[dev] > 0 ? sm_counts[dev] : 1;
+    const int sms = sm_count(dev);
     const int ctas = tiles < sms ? tiles : (sms < kMaxCtas ? sms : kMaxCtas);
     if (indices) cudaMemcpyAsync(idx, indices, (size_t)batch * 8, cudaMemcpyDeviceToDevice, s);
     else replay_sample_kernel<<<(batch + 255) / 256, 256, 0, s>>>(count, batch, keys, (uint64_t)update_index, idx);
@@ -710,9 +708,7 @@ int mr_ddpg_gradients(const mr_ddpg_state* st, const mr_replay* rb, int64_t coun
     int64_t* idx = (int64_t*)workspace;
     float* slabs = (float*)((char*)workspace + (((int64_t)batch * 8 + 63) / 64) * 64);
     const int tiles = (batch + kTile - 1) / kTile;
-    static int sm_counts[kMaxDevices] = {};
-    if (!sm_counts[dev]) cudaDeviceGetAttribute(&sm_counts[dev], cudaDevAttrMultiProcessorCount, dev);
-    const int sms = sm_counts[dev] > 0 ? sm_counts[dev] : 1;
+    const int sms = sm_count(dev);
     const int ctas = tiles < sms ? tiles : (sms < kMaxCtas ? sms : kMaxCtas);
     // the same rows for the critic and the actor call of one update: given, or regenerated from (seed, update_index)
     if (indices) cudaMemcpyAsync(idx, indices, (size_t)batch * 8, cudaMemcpyDeviceToDevice, s);

@@ -153,15 +153,12 @@ static void launch_kq_mean(const double* q, int64_t n_q, const mr_gp_model* gp, 
     const bool aligned = (((uintptr_t)gp->x_train_scaled | (uintptr_t)gp->alpha) & 15u) == 0;   // TMA bulk copies
     if (smem <= 200 * 1024 && aligned) {
         constexpr int QPW = 4;
-        static int sms[kMaxDevices] = {};
-        const int dev = current_device();
-        if (!sms[dev]) { cudaDeviceGetAttribute(&sms[dev], cudaDevAttrMultiProcessorCount, dev); if (sms[dev] <= 0) sms[dev] = 148; }
         cudaFuncSetAttribute(gp_kq_mean_smem_kernel<DIM, WRITE_KQ, QPW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         int per_sm = (int)((220 * 1024) / (smem + 1024));
         if (per_sm < 1) per_sm = 1;
         if (per_sm > 4) per_sm = 4;
         int64_t want = (n_q + 8 * QPW - 1) / (8 * QPW);             // CTAs needed if every warp took one pass
-        int64_t grid = (int64_t)sms[dev] * per_sm;
+        int64_t grid = (int64_t)sm_count(current_device()) * per_sm;
         if (grid > want) grid = want;
         if (grid < 1) grid = 1;
         gp_kq_mean_smem_kernel<DIM, WRITE_KQ, QPW><<<(unsigned)grid, 256, smem, s>>>(q, n_q, gp->x_train_scaled, gp->alpha,
@@ -798,10 +795,9 @@ int mr_actor_forward_env(const float* actor, const void* obs, int64_t obs_row_st
     if (!ctas[dev]) {
         cudaFuncSetAttribute(actor_forward_tc_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ActorTcSmem));
         cudaFuncSetAttribute(actor_forward_tc_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(ActorTcSmem));
-        int sms = 0, occ = 0;
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        int occ = 0;
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, actor_forward_tc_kernel<double>, kTcRows, sizeof(ActorTcSmem));
-        ctas[dev] = (sms > 0 ? sms : 148) * (occ > 0 ? occ : 1);
+        ctas[dev] = sm_count(dev) * (occ > 0 ? occ : 1);
     }
     const int64_t tiles = (n + kTcRows - 1) / kTcRows;
     const unsigned grid = (unsigned)(tiles < ctas[dev] ? tiles : ctas[dev]);
