@@ -523,6 +523,39 @@ int mr_ddpg_apply(const mr_ddpg_state* st, int32_t which, const float* grad, dou
  * cycle-walked into [0, count).  indices_out: device int64 [batch]. */
 int mr_replay_sample(int64_t count, int32_t batch, uint64_t seed, int64_t update_index, int64_t* indices_out, void* stream);
 
+/* ---- DDPG populations: many independent learners trained in lockstep ------------------------------------------------
+ * Member p is a complete learner: its own parameters, targets, Adam moments, hyper-parameters, sampling seed and replay
+ * ring.  Every array is member-major: st.actor is [members][mr_actor_param_count()], st.critic and the other critic
+ * arrays [members][mr_critic_param_count()], ring.s [members][capacity][5], ring.a [members][capacity][2], ring.r and
+ * ring.d [members][capacity]; ring.capacity is the capacity of ONE member's ring.  The members share the ring count,
+ * the minibatch size and Adam's step count.  Member p of a population computes exactly what mr_ddpg_update (NULL
+ * workspace) and mr_env_rollout_ddpg_collect compute for that learner alone. */
+#define MR_DDPG_MAX_MEMBERS 256
+typedef struct mr_ddpg_population {
+    int32_t members;                  /* 1..MR_DDPG_MAX_MEMBERS                                              */
+    mr_ddpg_state st;                 /* every array [members][param count]                                  */
+    mr_replay ring;                   /* every array [members][capacity][...]; capacity is per member        */
+    const mr_ddpg_hyper* hyper;       /* HOST [members]                                                      */
+    const uint64_t* seeds;            /* HOST [members]: the sampling seed of each member (mr_ddpg_update's)  */
+} mr_ddpg_population;
+
+/* mr_ddpg_update (single-CTA kernel, kernel-sampled minibatch) for every member in ONE launch, one CTA per member:
+ * member p samples `batch` of its first `count` ring rows with seeds[p] and update_index, and updates its own state with
+ * hyper[p].  batch in 1..4096, batch <= count <= capacity.  info_out: device [members][2] (critic loss, mean Q) or NULL.
+ * The hyper-parameters and seeds are read on the host during the call. */
+int mr_ddpg_update_population(const mr_ddpg_population* pop, int64_t count, int32_t batch, int64_t update_index,
+                              float* info_out, void* stream);
+
+/* mr_env_rollout_ddpg_collect for a population: n = members x N envs, N a positive multiple of 128; env p N + j acts
+ * with member p's actor io->actor + p mr_actor_param_count() and writes its transition (k, j) to member p's ring slot
+ * (head + k N + j) % capacity (c->ring as in mr_ddpg_population, N <= capacity).  The OU state and parameters cover all
+ * n envs (one process per env, as in mr_env_rollout_ddpg_collect); io->stats (or NULL) is [members][MR_STATS_LEN], one
+ * statistics row per member.  The caller advances head by K N (mod capacity), count to min(count + K N, capacity) and
+ * the OU counter by K. */
+int mr_env_rollout_ddpg_collect_population(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                                           const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
+                                           const mr_ddpg_collect* c, int32_t members, const mr_step_out* out, void* stream);
+
 /* mr_actor_forward for MR_Env observations — obs rows 2, 3 (the goal) are identically zero (MR_env.py:57) and are not
  * read — with the hidden layer on the tensor cores (tcgen05, 3xTF32 ~ fp32 accuracy).  Same arguments. */
 int mr_actor_forward_env(const float* actor, const void* obs, int64_t obs_row_stride, int64_t n, int32_t dtype,

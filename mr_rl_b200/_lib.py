@@ -104,6 +104,14 @@ class DDPGHyper(C.Structure):
                 ("action_bound", C.c_double * 2), ("adam_beta1", C.c_double), ("adam_beta2", C.c_double), ("adam_eps", C.c_double)]
 
 
+DDPG_MAX_MEMBERS = 256
+
+
+class DDPGPopulation(C.Structure):
+    _fields_ = [("members", C.c_int32), ("st", DDPGState), ("ring", Replay), ("hyper", C.POINTER(DDPGHyper)),
+                ("seeds", C.POINTER(C.c_uint64))]
+
+
 GP_PAD = 128
 
 
@@ -113,7 +121,8 @@ EXPORTS = ("mr_abi_version", "mr_last_error", "mr_default_params", "mr_fill_time
            "mr_learn_workspace_bytes", "mr_ddpg_workspace_bytes", "mr_replay_sample", "mr_actor_forward_env", "mr_ddpg_gradients", "mr_ddpg_apply", "mr_gp_correct_heading_cheb", "mr_host_pipeline_create", "mr_host_pipeline_destroy", "mr_env_step_host",
            "mr_actor_forward", "mr_set_step_path", "mr_env_reset_ex", "mr_counter_set", "mr_set_actor_path",
            "mr_host_register", "mr_host_unregister", "mr_philox_normals", "mr_gp_correct_action_2d",
-           "mr_env_rollout_gp_heading", "mr_env_rollout_ddpg_collect")
+           "mr_env_rollout_gp_heading", "mr_env_rollout_ddpg_collect", "mr_ddpg_update_population",
+           "mr_env_rollout_ddpg_collect_population")
 
 _lib = None
 
@@ -156,6 +165,12 @@ def load():
     lib.mr_env_rollout_ddpg_collect.argtypes = [P(EnvState), C.c_int64, C.c_int32, P(SimParams), P(Noise), P(TimeTable),
                                                 P(RolloutIO), P(DDPGCollect), P(StepOut), C.c_void_p]
     lib.mr_env_rollout_ddpg_collect.restype = C.c_int
+    lib.mr_env_rollout_ddpg_collect_population.argtypes = [P(EnvState), C.c_int64, C.c_int32, P(SimParams), P(Noise),
+                                                           P(TimeTable), P(RolloutIO), P(DDPGCollect), C.c_int32, P(StepOut),
+                                                           C.c_void_p]
+    lib.mr_env_rollout_ddpg_collect_population.restype = C.c_int
+    lib.mr_ddpg_update_population.argtypes = [P(DDPGPopulation), C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]
+    lib.mr_ddpg_update_population.restype = C.c_int
     lib.mr_gp_predict.argtypes = [P(GPModel), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                   C.c_void_p]
     lib.mr_gp_correct_heading.argtypes = [P(GPModel), P(GPModel), C.c_void_p, C.c_int64, C.c_double, C.c_double, C.c_double,

@@ -68,8 +68,8 @@ __device__ __forceinline__ void tc_split(float v, float& hi, float& lo) {
     lo = v - hi;                                               // exact; its leading bits feed the second pass
 }
 
-// once per CTA: parameters, W2 hi/lo in UMMA layout, TMEM allocation, mbarrier
-__device__ __forceinline__ void actor_tc_setup(ActorTcSmem& sm, const float* __restrict__ actor) {
+// the actor's parameters in shared memory: W2 hi/lo in UMMA layout, folded layer 1, epilogue constants
+__device__ __forceinline__ void actor_tc_stage(ActorTcSmem& sm, const float* __restrict__ actor) {
     const int tid = threadIdx.x;
     for (int idx = tid; idx < kActorHidden * kActorHidden; idx += kTcRows) {
         const int k = idx / kActorHidden, nn = idx % kActorHidden;      // W2[k][nn] (input-major)
@@ -93,6 +93,12 @@ __device__ __forceinline__ void actor_tc_setup(ActorTcSmem& sm, const float* __r
                                  actor[kOffW3 + tid * kActorOut], actor[kOffW3 + tid * kActorOut + 1]);
     }
     if (tid < 2) sm.b3[tid] = actor[kOffB3 + tid];
+}
+
+// once per CTA: parameters, TMEM allocation, mbarrier
+__device__ __forceinline__ void actor_tc_setup(ActorTcSmem& sm, const float* __restrict__ actor) {
+    const int tid = threadIdx.x;
+    actor_tc_stage(sm, actor);
     if (tid < 32) {                                                    // one warp owns the TMEM allocation
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc_smem_u32(&sm.tmem_base)), "r"(64));
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
@@ -102,6 +108,17 @@ __device__ __forceinline__ void actor_tc_setup(ActorTcSmem& sm, const float* __r
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");       // b_hi / b_lo visible to the tensor core
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+}
+
+// another actor for the CTA's next tile (population collector).  Every thread has waited for the MMAs of its last
+// call, so the tensor core no longer reads the operands; the first barrier orders the epilogue's reads before the overwrite.
+__device__ __forceinline__ void actor_tc_restage(ActorTcSmem& sm, const float* __restrict__ actor) {
+    __syncthreads();
+    actor_tc_stage(sm, actor);
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");

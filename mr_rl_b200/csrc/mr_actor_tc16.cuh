@@ -151,8 +151,8 @@ __device__ __forceinline__ void t16_ld16(uint32_t taddr, uint32_t (&r)[16]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// once per CTA: weights split into fp16 hi / lo in UMMA layout, folded BN constants, TMEM allocation, mbarriers
-__device__ __forceinline__ void actor_tc16_setup(ActorTc16Smem& sm, const float* __restrict__ actor) {
+// weights split into fp16 hi / lo in UMMA layout, folded BN constants
+__device__ __forceinline__ void actor_tc16_stage(ActorTc16Smem& sm, const float* __restrict__ actor) {
     const int tid = threadIdx.x;
     char* b2h = reinterpret_cast<char*>(sm.b2_hi);
     char* b2l = reinterpret_cast<char*>(sm.b2_lo);
@@ -189,6 +189,12 @@ __device__ __forceinline__ void actor_tc16_setup(ActorTc16Smem& sm, const float*
         e[0] = s2; e[2] = t2; e[4] = actor[kOffW3 + tid * kActorOut]; e[6] = actor[kOffW3 + tid * kActorOut + 1];
     }
     if (tid < 2) sm.b3[tid] = actor[kOffB3 + tid];
+}
+
+// once per CTA: the weights, TMEM allocation, mbarriers
+__device__ __forceinline__ void actor_tc16_setup(ActorTc16Smem& sm, const float* __restrict__ actor) {
+    const int tid = threadIdx.x;
+    actor_tc16_stage(sm, actor);
     if (tid < 32) {                                                    // one warp owns the TMEM allocation
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(t16_smem_u32(&sm.tmem_base)), "r"(kT16Cols));
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
@@ -203,6 +209,18 @@ __device__ __forceinline__ void actor_tc16_setup(ActorTc16Smem& sm, const float*
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");       // weights visible to the tensor core
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+}
+
+// another actor for the persistent CTA's next tile (population collector).  Every thread has waited for the MMAs of its
+// last call, so the tensor core no longer reads the operands; the first barrier orders the epilogue's reads before the
+// overwrite.  TMEM, mbarriers and descriptors stay.
+__device__ __forceinline__ void actor_tc16_restage(ActorTc16Smem& sm, const float* __restrict__ actor) {
+    __syncthreads();
+    actor_tc16_stage(sm, actor);
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");

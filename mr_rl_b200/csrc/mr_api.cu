@@ -612,13 +612,13 @@ extern "C" int mr_env_rollout_gp_heading(const mr_env_state* st, int64_t n, int3
                            : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, &gh, nullptr, out, s);
 }
 
-extern "C" int mr_env_rollout_ddpg_collect(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
-                                           const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
-                                           const mr_ddpg_collect* c, const mr_step_out* out, void* stream) {
-    mr::NvtxRange nvtx_range("mr_env_rollout_ddpg_collect");
-    using mr::fail;
-    const char* fn = "mr_env_rollout_ddpg_collect";
-    int rc = mr::check_rollout(fn, st, n, dtype, p, nz, io, out);
+namespace mr {
+// the checks of mr_env_rollout_ddpg_collect, and its CollectView; ring_envs: the envs that write into one ring (n, or a
+// population member's N), described by `what` in the error message
+static int collect_view(const char* fn, const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                        const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io, const mr_ddpg_collect* c,
+                        const mr_step_out* out, int64_t ring_envs, const char* what, CollectView& cv) {
+    int rc = check_rollout(fn, st, n, dtype, p, nz, io, out);
     if (rc) return rc;
     if (io->action_source != MR_ACTIONS_ACTOR)
         return fail(MR_ERR_ARG, "%s: io->action_source must be MR_ACTIONS_ACTOR (%d), got %d", fn, MR_ACTIONS_ACTOR, io->action_source);
@@ -630,22 +630,58 @@ extern "C" int mr_env_rollout_ddpg_collect(const mr_env_state* st, int64_t n, in
     if (!out || !out->obs) return fail(MR_ERR_ARG, "%s: the observation rows out->obs (the first policy input) are required", fn);
     if (rb.capacity <= 0) return fail(MR_ERR_ARG, "%s: ring capacity must be positive", fn);
     if (c->head < 0 || c->head >= rb.capacity) return fail(MR_ERR_ARG, "%s: need 0 <= head < capacity", fn);
-    if (n > rb.capacity) return fail(MR_ERR_ARG, "%s: more envs than the ring holds (n > capacity)", fn);
+    if (ring_envs > rb.capacity) return fail(MR_ERR_ARG, "%s: %s", fn, what);
     for (double v : {c->ou_theta, c->ou_mu, c->ou_sigma, c->ou_dt})
         if (!std::isfinite(v)) return fail(MR_ERR_ARG, "%s: ou_theta, ou_mu, ou_sigma and ou_dt must be finite", fn);
     if (!tt || !tt->t || tt->len < 2) return fail(MR_ERR_ARG, "%s: time table missing", fn);
     if (st->a0) return fail(MR_ERR_UNSUPPORTED, "%s: the collector does not take per-env parameter rows", fn);
-    if (mr::g_actor_path == 1) return fail(MR_ERR_UNSUPPORTED, "%s: the CUDA-core actor path (mr_set_actor_path(1)) has no collector", fn);
-    if (n == 0 || io->k_steps == 0) return MR_OK;
-    const mr::Params pp = mr::to_params(*p, nz);
-    const mr::TimeView tv{tt->t, tt->len};
-    mr::CollectView cv;
+    if (g_actor_path == 1) return fail(MR_ERR_UNSUPPORTED, "%s: the CUDA-core actor path (mr_set_actor_path(1)) has no collector", fn);
     cv.ou = c->ou_state;
-    mr::philox_make_keys(c->ou_seed, cv.keys);
+    philox_make_keys(c->ou_seed, cv.keys);
     cv.theta = c->ou_theta; cv.mu = c->ou_mu; cv.sd = c->ou_sigma * sqrt(c->ou_dt); cv.dt = c->ou_dt;
     cv.counter = c->ou_counter; cv.env_base = c->ou_env_base;
     cv.s = rb.s; cv.a = rb.a; cv.r = rb.r; cv.d = rb.d; cv.s2 = rb.s2;
     cv.capacity = rb.capacity; cv.head = c->head;
+    cv.member_envs = 0;
+    return MR_OK;
+}
+}  // namespace mr
+
+extern "C" int mr_env_rollout_ddpg_collect(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                                           const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
+                                           const mr_ddpg_collect* c, const mr_step_out* out, void* stream) {
+    mr::NvtxRange nvtx_range("mr_env_rollout_ddpg_collect");
+    mr::CollectView cv;
+    int rc = mr::collect_view("mr_env_rollout_ddpg_collect", st, n, dtype, p, nz, tt, io, c, out, n,
+                              "more envs than the ring holds (n > capacity)", cv);
+    if (rc) return rc;
+    if (n == 0 || io->k_steps == 0) return MR_OK;
+    const mr::Params pp = mr::to_params(*p, nz);
+    const mr::TimeView tv{tt->t, tt->len};
+    cudaStream_t s = (cudaStream_t)stream;
+    return dtype == MR_F64 ? mr::do_rollout<double>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s)
+                           : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s);
+}
+
+extern "C" int mr_env_rollout_ddpg_collect_population(const mr_env_state* st, int64_t n, int32_t dtype, const mr_sim_params* p,
+                                                      const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
+                                                      const mr_ddpg_collect* c, int32_t members, const mr_step_out* out,
+                                                      void* stream) {
+    mr::NvtxRange nvtx_range("mr_env_rollout_ddpg_collect_population");
+    using mr::fail;
+    const char* fn = "mr_env_rollout_ddpg_collect_population";
+    if (members < 1 || members > MR_DDPG_MAX_MEMBERS) return fail(MR_ERR_ARG, "%s: members must be in 1..%d", fn, MR_DDPG_MAX_MEMBERS);
+    // the tensor-core actor multiplies a whole 128-env tile by one weight matrix: a tile must not span two members
+    if (n <= 0 || n % members != 0 || (n / members) % 128 != 0)
+        return fail(MR_ERR_ARG, "%s: n must be members x N with N a positive multiple of 128", fn);
+    mr::CollectView cv;
+    int rc = mr::collect_view(fn, st, n, dtype, p, nz, tt, io, c, out, n / members,
+                              "more envs per member than its ring holds (N > capacity)", cv);
+    if (rc) return rc;
+    cv.member_envs = n / members;
+    if (io->k_steps == 0) return MR_OK;
+    const mr::Params pp = mr::to_params(*p, nz);
+    const mr::TimeView tv{tt->t, tt->len};
     cudaStream_t s = (cudaStream_t)stream;
     return dtype == MR_F64 ? mr::do_rollout<double>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s)
                            : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s);

@@ -270,9 +270,10 @@ struct CollectView {
     uint64_t counter, env_base;     // step k draws OU sample counter + k of env env_base + i
     float *s, *a, *r, *d, *s2;      // ring rows [capacity][5] / [capacity][2] / [capacity] / [capacity] / [capacity][5]
     int64_t capacity, head;         // transition (k, i) goes to slot (head + k n + i) % capacity
+    int64_t member_envs;            // population (mr_env_rollout_ddpg_collect_population): envs per member N; 0: one learner
 };
 // The fused rollout of every action source.  gh: the GP heading policy, only from mr_env_rollout_gp_heading; cv: the
-// DDPG collector, only from mr_env_rollout_ddpg_collect; both null from mr_env_rollout.
+// DDPG collector, only from mr_env_rollout_ddpg_collect(_population); both null from mr_env_rollout.
 template <class T, int MODE>
 int launch_rollout(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
                    const TimeView& tv, const Params& p, int64_t n, const GpHeadingView* gh, const CollectView* cv,

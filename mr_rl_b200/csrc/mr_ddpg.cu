@@ -13,6 +13,9 @@
 // moving statistics (oracle/ddpg_oracle.py states this; parity unpinned — no TensorFlow in this image).
 #include <cuda_runtime.h>
 
+#include <cmath>
+#include <initializer_list>
+
 #include "mr_actor.cuh"
 #include "mr_common.cuh"
 #include "mr_ou.cuh"
@@ -301,14 +304,19 @@ __device__ void actor_tile(DdpgSmem& sm, int nb, bool acc, float inv_b, const Dd
     fc_bwd_w(sm.S, 5, sm.G1, kLd64, nb, 5, 64, ga + kOffW1, ga + kOffB1, acc);
 }
 
-__global__ void __launch_bounds__(kDdpgThreads, 1)
-ddpg_update_kernel(float* __restrict__ actor, float* __restrict__ actor_t, float* __restrict__ critic, float* __restrict__ critic_t,
-                   float* __restrict__ am, float* __restrict__ av, float* __restrict__ cm, float* __restrict__ cv,
-                   float* __restrict__ ga, float* __restrict__ gc,
-                   const float* __restrict__ rs, const float* __restrict__ ra, const float* __restrict__ rr,
-                   const float* __restrict__ rd, const float* __restrict__ rs2, int64_t count, int batch,
-                   const int64_t* __restrict__ indices, PhiloxKeys keys, uint64_t update_index, DdpgHyper h,
-                   float* __restrict__ info_out) {
+// One learner update by the whole CTA: the body of ddpg_update_kernel (one learner) and of ddpg_update_population_kernel
+// (member blockIdx.x of a population).  Member p of a population must compute what the solo kernel computes bit for bit,
+// which holds only while ptxas schedules and contracts the float arithmetic of both inlined copies alike: hand the body
+// h and keys in registers (as the population kernel does) and check with test_population_update_equals_solo_updates
+// (tests/test_ddpg_population.py) after any change here or to the compiler.
+__device__ __forceinline__ void ddpg_update_cta(float* __restrict__ actor, float* __restrict__ actor_t, float* __restrict__ critic,
+                                                float* __restrict__ critic_t, float* __restrict__ am, float* __restrict__ av,
+                                                float* __restrict__ cm, float* __restrict__ cv, float* __restrict__ ga,
+                                                float* __restrict__ gc, const float* __restrict__ rs, const float* __restrict__ ra,
+                                                const float* __restrict__ rr, const float* __restrict__ rd,
+                                                const float* __restrict__ rs2, int64_t count, int batch,
+                                                const int64_t* __restrict__ indices, const PhiloxKeys& keys, uint64_t update_index,
+                                                const DdpgHyper& h, float* __restrict__ info_out) {
     extern __shared__ __align__(16) unsigned char ddpg_smem_raw[];
     DdpgSmem& sm = *reinterpret_cast<DdpgSmem*>(ddpg_smem_raw);
     const int tid = threadIdx.x;
@@ -383,6 +391,41 @@ ddpg_update_kernel(float* __restrict__ actor, float* __restrict__ actor_t, float
         critic_t[k] = h.tau * critic[k] + (1.f - h.tau) * critic_t[k];
     }
     if (tid == 0 && info_out) { info_out[0] = loss_acc * inv_b; info_out[1] = q_acc * inv_b; }
+}
+
+__global__ void __launch_bounds__(kDdpgThreads, 1)
+ddpg_update_kernel(float* __restrict__ actor, float* __restrict__ actor_t, float* __restrict__ critic, float* __restrict__ critic_t,
+                   float* __restrict__ am, float* __restrict__ av, float* __restrict__ cm, float* __restrict__ cv,
+                   float* __restrict__ ga, float* __restrict__ gc,
+                   const float* __restrict__ rs, const float* __restrict__ ra, const float* __restrict__ rr,
+                   const float* __restrict__ rd, const float* __restrict__ rs2, int64_t count, int batch,
+                   const int64_t* __restrict__ indices, PhiloxKeys keys, uint64_t update_index, DdpgHyper h,
+                   float* __restrict__ info_out) {
+    ddpg_update_cta(actor, actor_t, critic, critic_t, am, av, cm, cv, ga, gc, rs, ra, rr, rd, rs2, count, batch, indices, keys,
+                    update_index, h, info_out);
+}
+
+// ---- a population of independent learners (mr_ddpg_update_population): one CTA per member, every array member-major.
+//      The members' hyper-parameters and sampling keys travel in the launch's parameter space (no device buffer, no copy).
+constexpr int kMaxMembers = MR_DDPG_MAX_MEMBERS;
+struct DdpgMember { DdpgHyper h; PhiloxKeys keys; };
+struct DdpgMembers { DdpgMember m[kMaxMembers]; };             // 29.7 KB: kernel parameters may take 32 KB (CUDA 12.1+)
+static_assert(sizeof(DdpgMembers) < 31 * 1024, "the members must fit the kernel parameter space next to the pointers");
+struct DdpgStack {                                              // mr_ddpg_state + mr_replay of the population
+    float *actor, *actor_t, *critic, *critic_t, *am, *av, *cm, *cv, *ga, *gc;
+    const float *rs, *ra, *rr, *rd, *rs2;
+    int64_t capacity;
+};
+
+__global__ void __launch_bounds__(kDdpgThreads, 1)
+ddpg_update_population_kernel(DdpgStack ps, int64_t count, int batch, uint64_t update_index, float* __restrict__ info_out,
+                              const __grid_constant__ DdpgMembers mem) {
+    const int64_t p = blockIdx.x, pa = p * kActorParams, pc = p * kCriticParams, row = p * ps.capacity;
+    const DdpgHyper h = mem.m[p].h;                              // in registers, as the solo kernel's parameters: the
+    const PhiloxKeys keys = mem.m[p].keys;                       // compiler then hoists and contracts the same way
+    ddpg_update_cta(ps.actor + pa, ps.actor_t + pa, ps.critic + pc, ps.critic_t + pc, ps.am + pa, ps.av + pa, ps.cm + pc,
+                    ps.cv + pc, ps.ga + pa, ps.gc + pc, ps.rs + row * 5, ps.ra + row * 2, ps.rr + row, ps.rd + row,
+                    ps.rs2 + row * 5, count, batch, nullptr, keys, update_index, h, info_out ? info_out + 2 * p : nullptr);
 }
 
 // =====================================================================================================================
@@ -561,6 +604,14 @@ __global__ void ou_noise_kernel(double* __restrict__ x, T* __restrict__ actions,
 
 }  // namespace mr
 
+namespace mr {
+// the floats every update kernel sees: (float) of each double of mr_ddpg_hyper
+static DdpgHyper to_hyper(const mr_ddpg_hyper& hp) {
+    return DdpgHyper{(float)hp.gamma, (float)hp.tau, (float)hp.lr_actor, (float)hp.lr_critic, (float)hp.action_bound[0],
+                     (float)hp.action_bound[1], (float)hp.adam_beta1, (float)hp.adam_beta2, (float)hp.adam_eps};
+}
+}  // namespace mr
+
 extern "C" {
 
 int32_t mr_critic_param_count(void) { return mr::kCriticParams; }
@@ -636,8 +687,7 @@ int mr_ddpg_update(const mr_ddpg_state* st, const mr_replay* rb, int64_t count, 
         return fail(MR_ERR_ARG, "mr_ddpg_update: batch must be in 1..%d (larger ones need the workspace of mr_ddpg_workspace_bytes)", kMaxBatch);
     if (count < batch || count > rb->capacity) return fail(MR_ERR_ARG, "mr_ddpg_update: need batch <= count <= capacity (the reference waits for min_batch transitions)");
     if (update_index < 1) return fail(MR_ERR_ARG, "mr_ddpg_update: update_index is Adam's step count, starting at 1");
-    DdpgHyper h{(float)hp->gamma, (float)hp->tau, (float)hp->lr_actor, (float)hp->lr_critic, (float)hp->action_bound[0],
-                (float)hp->action_bound[1], (float)hp->adam_beta1, (float)hp->adam_beta2, (float)hp->adam_eps};
+    const DdpgHyper h = to_hyper(*hp);
     PhiloxKeys keys;
     philox_make_keys(seed, keys);
     cudaStream_t s = (cudaStream_t)stream;
@@ -680,6 +730,47 @@ int mr_ddpg_update(const mr_ddpg_state* st, const mr_replay* rb, int64_t count, 
     return check_launch("mr_ddpg_update");
 }
 
+int mr_ddpg_update_population(const mr_ddpg_population* pop, int64_t count, int32_t batch, int64_t update_index, float* info_out,
+                              void* stream) {
+    mr::NvtxRange nvtx_range("mr_ddpg_update_population");
+    using namespace mr;
+    const char* fn = "mr_ddpg_update_population";
+    if (!pop) return fail(MR_ERR_ARG, "%s: null population", fn);
+    if (pop->members < 1 || pop->members > kMaxMembers) return fail(MR_ERR_ARG, "%s: members must be in 1..%d", fn, kMaxMembers);
+    const mr_ddpg_state* st = &pop->st;
+    if (!st->actor || !st->actor_target || !st->critic || !st->critic_target || !st->adam_actor_m || !st->adam_actor_v ||
+        !st->adam_critic_m || !st->adam_critic_v || !st->grad_actor || !st->grad_critic)
+        return fail(MR_ERR_ARG, "%s: null learner state", fn);
+    const mr_replay* rb = &pop->ring;
+    if (!rb->s || !rb->a || !rb->r || !rb->d || !rb->s2) return fail(MR_ERR_ARG, "%s: null replay ring array", fn);
+    if (!pop->hyper) return fail(MR_ERR_ARG, "%s: null hyper-parameters", fn);
+    if (!pop->seeds) return fail(MR_ERR_ARG, "%s: null seeds", fn);
+    if (batch <= 0 || batch > kMaxBatch) return fail(MR_ERR_ARG, "%s: batch must be in 1..%d", fn, kMaxBatch);
+    if (count < batch || count > rb->capacity) return fail(MR_ERR_ARG, "%s: need batch <= count <= capacity", fn);
+    if (update_index < 1) return fail(MR_ERR_ARG, "%s: update_index is Adam's step count, starting at 1", fn);
+    DdpgMembers mem{};                                            // rows past `members` are not read
+    for (int p = 0; p < pop->members; ++p) {
+        const mr_ddpg_hyper& hp = pop->hyper[p];
+        for (double v : {hp.gamma, hp.tau, hp.lr_actor, hp.lr_critic, hp.action_bound[0], hp.action_bound[1], hp.adam_beta1,
+                         hp.adam_beta2, hp.adam_eps})
+            if (!std::isfinite(v)) return fail(MR_ERR_ARG, "%s: hyper-parameters of member %d must be finite", fn, p);
+        mem.m[p].h = to_hyper(hp);
+        philox_make_keys(pop->seeds[p], mem.m[p].keys);
+    }
+    const DdpgStack ps{st->actor, st->actor_target, st->critic, st->critic_target, st->adam_actor_m, st->adam_actor_v,
+                       st->adam_critic_m, st->adam_critic_v, st->grad_actor, st->grad_critic, rb->s, rb->a, rb->r, rb->d, rb->s2,
+                       rb->capacity};
+    static bool attr[kMaxDevices] = {};
+    const int dev = current_device();
+    if (!attr[dev]) {
+        cudaFuncSetAttribute(ddpg_update_population_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DdpgSmem));
+        attr[dev] = true;
+    }
+    ddpg_update_population_kernel<<<pop->members, kDdpgThreads, sizeof(DdpgSmem), (cudaStream_t)stream>>>(
+        ps, count, batch, (uint64_t)update_index, info_out, mem);
+    return check_launch(fn);
+}
+
 int mr_ddpg_gradients(const mr_ddpg_state* st, const mr_replay* rb, int64_t count, int32_t batch, const int64_t* indices,
                       uint64_t seed, int64_t update_index, const mr_ddpg_hyper* hp, int32_t which, float* grad_out,
                       void* workspace, int64_t workspace_bytes, void* stream) {
@@ -693,8 +784,7 @@ int mr_ddpg_gradients(const mr_ddpg_state* st, const mr_replay* rb, int64_t coun
     if (count < batch || count > rb->capacity) return fail(MR_ERR_ARG, "mr_ddpg_gradients: need batch <= count <= capacity");
     if (!workspace || workspace_bytes < mr_ddpg_workspace_bytes(batch)) return fail(MR_ERR_ARG, "mr_ddpg_gradients: workspace too small");
     if ((uintptr_t)workspace & 15u) return fail(MR_ERR_ARG, "mr_ddpg_gradients: workspace must be 16-byte aligned");
-    DdpgHyper h{(float)hp->gamma, (float)hp->tau, (float)hp->lr_actor, (float)hp->lr_critic, (float)hp->action_bound[0],
-                (float)hp->action_bound[1], (float)hp->adam_beta1, (float)hp->adam_beta2, (float)hp->adam_eps};
+    const DdpgHyper h = to_hyper(*hp);
     PhiloxKeys keys;
     philox_make_keys(seed, keys);
     cudaStream_t s = (cudaStream_t)stream;
@@ -735,8 +825,7 @@ int mr_ddpg_apply(const mr_ddpg_state* st, int32_t which, const float* grad, dou
     if (!hp || !grad) return fail(MR_ERR_ARG, "mr_ddpg_apply: null argument");
     if (which != 0 && which != 1) return fail(MR_ERR_ARG, "mr_ddpg_apply: which must be 0 (critic) or 1 (actor)");
     if (update_index < 1) return fail(MR_ERR_ARG, "mr_ddpg_apply: update_index is Adam's step count, starting at 1");
-    DdpgHyper h{(float)hp->gamma, (float)hp->tau, (float)hp->lr_actor, (float)hp->lr_critic, (float)hp->action_bound[0],
-                (float)hp->action_bound[1], (float)hp->adam_beta1, (float)hp->adam_beta2, (float)hp->adam_eps};
+    const DdpgHyper h = to_hyper(*hp);
     const float t = (float)update_index;
     const float corr = sqrtf(1.f - powf(h.beta2, t)) / (1.f - powf(h.beta1, t));
     cudaStream_t s = (cudaStream_t)stream;

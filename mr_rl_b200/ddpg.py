@@ -4,6 +4,8 @@ Mirrors the reference's pieces with the same names and arguments where they exis
 ``ReplayBuffer`` (:16-56) as a ring in HBM, ``OUNoise`` (:58-78) with one process per env, ``DDPGLearner`` = the
 ActorNetwork / CriticNetwork pair (:80-231) with their Adam optimisers and target networks, and ``train`` (:233-323)
 as a vectorised acting / learning loop.  One learner update (:285-305) is ONE kernel launch (csrc/mr_ddpg.cu).
+``DDPGPopulation`` / ``PopulationReplay`` / ``train_population`` train many independent learners (seeds, sweeps) with one
+update launch and one collect launch for all of them.
 Everything here fails without the CUDA library: there is no CPU path.
 """
 from __future__ import annotations
@@ -356,4 +358,206 @@ def _train_collect(env, learner, actor_noise, buffer_size, min_batch, steps, upd
         if log_every and (it + 1) % log_every == 0:
             row = log[it].cpu().numpy()
             print(f"launch {it + 1}/{launches} ({done} steps): mean reward {row[0]:.3f} critic loss {row[1]:.4g} mean Q {row[2]:.4g}")
+    return log.cpu().numpy()
+
+
+# ---- populations: many independent learners trained in lockstep -------------------------------------------------------
+# Member p of a population computes exactly what its solo run computes: DDPGLearner(seed=seeds[p], ...) with its own
+# ReplayBuffer, OUNoise(N, seed, env_base=p N) and VecMREnv(N, seed, env_base=p N) (env p N + j of the population's
+# VecMREnv(P N, seed) is env j of that solo env).  The difference is the launches: one update launch (one CTA per member)
+# and one collect launch for all members, where solo runs take P of each.
+
+def _per_member(name, v, members):
+    """A scalar for every member, or one value per member."""
+    if np.ndim(v) == 0:
+        return [float(v)] * members
+    v = [float(x) for x in v]
+    if len(v) != members:
+        raise ValueError(f"{name} has {len(v)} values for {members} members")
+    return v
+
+
+def _check_members(members):
+    members = int(members)
+    if not 1 <= members <= L.DDPG_MAX_MEMBERS:
+        raise ValueError(f"members must be in 1..{L.DDPG_MAX_MEMBERS}")
+    return members
+
+
+class PopulationReplay:
+    """One replay ring per member, stacked: ``s`` [P, buffer_size, 5], ``a`` [P, buffer_size, 2], ``r`` / ``d``
+    [P, buffer_size], ``s2`` [P, buffer_size, 5].  The members fill at the same rate, so ``head`` and ``count`` are shared.
+    ``random_seeds`` (a scalar or one per member) plays ReplayBuffer's ``random_seed``."""
+
+    def __init__(self, members, buffer_size, random_seeds=0, device="cuda"):
+        self.members = _check_members(members)
+        self.random_seeds = [int(s) for s in _per_member("random_seeds", random_seeds, self.members)]
+        self.lib = L.load()
+        self.device = _cuda_device(device)
+        self.buffer_size = int(buffer_size)
+        self.count = 0
+        self.head = 0
+        P, cap = self.members, self.buffer_size
+        z = lambda *s: torch.zeros(*s, dtype=torch.float32, device=self.device)
+        self.s, self.a, self.r, self.d, self.s2 = z(P, cap, 5), z(P, cap, 2), z(P, cap), z(P, cap), z(P, cap, 5)
+        self._c = L.Replay(self.s.data_ptr(), self.a.data_ptr(), self.r.data_ptr(), self.d.data_ptr(), self.s2.data_ptr(), cap)
+
+    def size(self):
+        return self.count
+
+    def member(self, p):
+        """Member p's ring as a ReplayBuffer whose arrays are views into the stacked rings; head and count are copied
+        from the population at this call."""
+        rb = ReplayBuffer.__new__(ReplayBuffer)
+        rb.lib, rb.device, rb.buffer_size, rb.random_seed = self.lib, self.device, self.buffer_size, self.random_seeds[p]
+        rb.count, rb.head = self.count, self.head
+        rb.s, rb.a, rb.r, rb.d, rb.s2 = self.s[p], self.a[p], self.r[p], self.d[p], self.s2[p]
+        rb._c = L.Replay(rb.s.data_ptr(), rb.a.data_ptr(), rb.r.data_ptr(), rb.d.data_ptr(), rb.s2.data_ptr(), rb.buffer_size)
+        return rb
+
+    def clear(self):
+        self.count = 0
+        self.head = 0
+
+
+class DDPGPopulation:
+    """``members`` independent DDPG learners in stacked storage: ``actor`` / ``actor_target`` [P, actor count], ``critic`` /
+    ``critic_target`` [P, critic count], and the Adam moments alike.  Member p starts exactly as
+    ``DDPGLearner(seed=seeds[p], actor_lr=..., ...)`` would.  ``actor_lr``, ``critic_lr``, ``tau`` and ``gamma`` are a
+    scalar or one value per member; ``action_bound`` is the env's action range, one pair for all.  ``stats`` [P, 8]
+    collects each member's episode statistics (``collect_population``)."""
+
+    def __init__(self, members, seeds=None, actor_lr=1e-3, critic_lr=1e-2, tau=1e-3, gamma=0.99,
+                 action_bound=(20.0, 2 * math.pi), target_init="independent", device="cuda"):
+        P = self.members = _check_members(members)
+        self.seeds = list(range(P)) if seeds is None else [int(s) for s in seeds]
+        if len(self.seeds) != P:
+            raise ValueError(f"seeds has {len(self.seeds)} values for {P} members")
+        hp = [_per_member(k, v, P) for k, v in (("actor_lr", actor_lr), ("critic_lr", critic_lr), ("tau", tau), ("gamma", gamma))]
+        self.lib = L.load()
+        self.device = _cuda_device(device)
+        learners = [DDPGLearner(action_bound=action_bound, actor_lr=hp[0][p], critic_lr=hp[1][p], tau=hp[2][p], gamma=hp[3][p],
+                                seed=self.seeds[p], device=self.device, target_init=target_init) for p in range(P)]
+        stack = lambda get: torch.stack([get(m) for m in learners]).contiguous()
+        self.actor, self.actor_target = stack(lambda m: m.actor), stack(lambda m: m.actor_target)
+        self.critic, self.critic_target = stack(lambda m: m.critic), stack(lambda m: m.critic_target)
+        self._moments = [stack(lambda m, i=i: m._moments[i]) for i in range(4)]
+        self._grads = [stack(lambda m, i=i: m._grads[i]) for i in range(2)]
+        for p, m in enumerate(learners):             # the members now work on views of the stacked storage
+            m.actor, m.actor_target, m.critic, m.critic_target = self.actor[p], self.actor_target[p], self.critic[p], self.critic_target[p]
+            m._moments = [t[p] for t in self._moments]
+            m._grads = [t[p] for t in self._grads]
+            m._c = L.DDPGState(m.actor.data_ptr(), m.actor_target.data_ptr(), m.critic.data_ptr(), m.critic_target.data_ptr(),
+                               *[t.data_ptr() for t in m._moments], *[t.data_ptr() for t in m._grads])
+        self._learners = learners
+        self.action_bound = learners[0].action_bound
+        self.hyper = (L.DDPGHyper * P)(*[m.hyper for m in learners])
+        state = L.DDPGState(self.actor.data_ptr(), self.actor_target.data_ptr(), self.critic.data_ptr(), self.critic_target.data_ptr(),
+                            *[t.data_ptr() for t in self._moments], *[t.data_ptr() for t in self._grads])
+        self._c = L.DDPGPopulation(P, state, L.Replay(), self.hyper, None)
+        self.updates = 0
+        self._info = torch.zeros(P, 2, dtype=torch.float32, device=self.device)
+        self.stats = torch.zeros(P, L.STATS_LEN, dtype=torch.float64, device=self.device)
+        self.kernel_launches = 0
+
+    def member(self, p):
+        """Member p as a DDPGLearner whose tensors are views into the population's storage (predict, actor_params,
+        critic_params and a solo update work on it).  Its update count is the population's at this call."""
+        m = self._learners[p]
+        m.updates = self.updates
+        return m
+
+    def update(self, replay, batch_size=64):
+        """One update of every member in ONE launch (one CTA per member): member p samples ``batch_size`` rows of its own
+        ring, as DDPGLearner.update does with ``seed ^ random_seed``, and takes the single-CTA update (batch 1..4096).
+        Returns the device tensor [P, 2] of (critic loss, mean Q)."""
+        batch_size = int(batch_size)
+        if replay.members != self.members:
+            raise ValueError(f"the replay has {replay.members} members, the population {self.members}")
+        if not 1 <= batch_size <= 4096:
+            raise ValueError("batch_size must be in 1..4096 (the single-CTA update of each member)")
+        seeds = (C.c_uint64 * self.members)(*[(s ^ r) & (2**64 - 1) for s, r in zip(self.seeds, replay.random_seeds)])
+        self._seeds_c = seeds                      # kept alive for the call
+        self._c.ring, self._c.seeds = replay._c, seeds
+        self.updates += 1
+        with torch.cuda.device(self.device):
+            rc = self.lib.mr_ddpg_update_population(C.byref(self._c), replay.count, batch_size, self.updates,
+                                                    self._info.data_ptr(), _stream(self.device))
+        if rc:
+            self.updates -= 1
+        L.check(rc, "mr_ddpg_update_population")
+        self.kernel_launches += 1
+        return self._info
+
+
+def _member_envs(env, members):
+    n = env.num_envs
+    if n % members or (n // members) % 128:
+        raise ValueError(f"env.num_envs = {n} must be members ({members}) x N with N a multiple of 128")
+    return n // members
+
+
+def collect_population(env, pop, actor_noise, replay, k_steps, **rollout_kw):
+    """``collect`` for every member in ONE launch: ``env`` holds members x N envs (N a multiple of 128), env p N + j acts
+    with member p's online actor and writes its transitions into member p's ring; one OUNoise covers all envs.  Advances
+    ``replay.head`` / ``replay.count`` by K N transitions and ``actor_noise.calls`` by K, and adds each member's episode
+    statistics to ``pop.stats[p]``.  Member p's ring, OU rows and envs end exactly as ``collect`` leaves its solo run."""
+    k = int(k_steps)
+    P = pop.members
+    if k < 1:
+        raise ValueError("k_steps must be at least 1")
+    if replay.members != P:
+        raise ValueError(f"the replay has {replay.members} members, the population {P}")
+    N = _member_envs(env, P)
+    if N > replay.buffer_size:
+        raise ValueError(f"{N} envs per member add more transitions per step than a member's replay buffer holds ({replay.buffer_size})")
+    if actor_noise.x_prev.shape[0] < env.num_envs:
+        raise ValueError(f"the OU noise has {actor_noise.x_prev.shape[0]} processes for {env.num_envs} envs")
+    if tuple(pop.action_bound) != (env.params.action_high[0], env.params.action_high[1]):
+        raise ValueError("pop.action_bound must equal the env's action_space.high (the in-kernel actor scales by it)")
+    c = L.DDPGCollect(actor_noise.x_prev.data_ptr(), actor_noise.theta, actor_noise.mu, actor_noise.sigma, actor_noise.dt,
+                      actor_noise.seed & (2**64 - 1), actor_noise.calls, actor_noise.env_base, replay._c, replay.head)
+    res = env.rollout(policy=pop.actor, k_steps=k, ddpg_collect=c, ddpg_population=(P, pop.stats), **rollout_kw)
+    replay.head = (replay.head + k * N) % replay.buffer_size
+    replay.count = min(replay.count + k * N, replay.buffer_size)
+    actor_noise.calls += k
+    return res
+
+
+def train_population(env, pop, actor_noise, buffer_size=10000, min_batch=64, steps=1000, updates_per_step=1, replay=None,
+                     noise_var=1, a0=1, log_every=0, collect_steps=64):
+    """``train(collect_steps=K)`` for a population: per launch one ``collect_population`` of K env steps, then
+    K * ``updates_per_step`` population updates once the rings hold ``min_batch`` transitions.  Returns the log
+    [P, launches, 3]: per member the mean reward of the launch's transitions, and the loss and mean Q of its last update.
+    With ``min_batch`` <= 64 member p's run equals its solo ``train(collect_steps=K)`` (above 64 samples the solo update
+    takes the data-parallel path, the population the single-CTA one)."""
+    P = pop.members
+    k = int(collect_steps)
+    if k < 1:
+        raise ValueError("collect_steps must be at least 1")
+    N = _member_envs(env, P)
+    replay = replay if replay is not None else PopulationReplay(P, buffer_size, 0, device=env.device)
+    if replay.members != P:
+        raise ValueError(f"the replay has {replay.members} members, the population {P}")
+    if N > replay.buffer_size:
+        raise ValueError(f"{N} envs per member add more transitions per step than a member's replay buffer holds ({replay.buffer_size})")
+    env.reset(noise_var=noise_var, a0=a0)
+    launches = (steps + k - 1) // k
+    log = torch.zeros(P, launches, 3, dtype=torch.float64, device=env.device)
+    rew_sum = pop.stats[:, L.STAT_NAMES.index("sum_reward")]
+    done = 0
+    for it in range(launches):
+        kk = min(k, steps - done)
+        before = rew_sum.clone()
+        collect_population(env, pop, actor_noise, replay, kk)
+        log[:, it, 0] = (rew_sum - before) / (kk * N)
+        if replay.size() >= min_batch:
+            for _ in range(kk * updates_per_step):
+                info = pop.update(replay, min_batch)
+            log[:, it, 1:] = info.double()
+        done += kk
+        if log_every and (it + 1) % log_every == 0:
+            row = log[:, it].mean(0).cpu().numpy()
+            print(f"launch {it + 1}/{launches} ({done} steps), mean over {P} members: reward {row[0]:.3f} "
+                  f"critic loss {row[1]:.4g} mean Q {row[2]:.4g}")
     return log.cpu().numpy()

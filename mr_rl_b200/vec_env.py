@@ -524,7 +524,8 @@ class VecMREnv:
 
     # ---- fused K-step rollout: utils.run_sim (utils.py:43-61) / the DDPG acting loop --------------
     def rollout(self, actions=None, k_steps=None, policy=None, record=False, record_state_prime=False,
-                record_done=False, accumulate_stats=True, record_episodes=False, reset_init=None, ddpg_collect=None):
+                record_done=False, accumulate_stats=True, record_episodes=False, reset_init=None, ddpg_collect=None,
+                ddpg_population=None):
         """K env steps in ONE launch with the state held in registers.
 
         actions : [K, N, 2] per-env actions, or [K, 2] / [K, >=2] one action row for every env
@@ -542,12 +543,15 @@ class VecMREnv:
                   instead of sampling init_space.
         ddpg_collect : with an actor ``policy``, the ``_lib.DDPGCollect`` of ``ddpg.collect``: the launch also adds OU
                   noise to the actions and writes every transition into the replay ring (mr_env_rollout_ddpg_collect).
+        ddpg_population : with ``ddpg_collect``, ``(members, stats)`` of ``ddpg.collect_population``: ``policy`` is the
+                  stacked actors [members, count], the ring arrays are stacked per member, and the statistics accumulate
+                  into ``stats`` [members, 8] instead of the env's vector (mr_env_rollout_ddpg_collect_population).
         Returns dict(obs, rew, done[, xy [K,2,N], state_prime [K,2,N], done_traj [K,N]]).
         """
         if torch.cuda.current_device() != self._dev_index:
             with torch.cuda.device(self.device):
                 return self.rollout(actions, k_steps, policy, record, record_state_prime, record_done, accumulate_stats,
-                                    record_episodes, reset_init, ddpg_collect)
+                                    record_episodes, reset_init, ddpg_collect, ddpg_population)
         n = self.num_envs
         io = L.RolloutIO()
         keep = []
@@ -571,7 +575,8 @@ class VecMREnv:
             k = int(k_steps)
         elif torch.is_tensor(policy):
             w = policy.to(device=self.device, dtype=torch.float32).contiguous()
-            if w.numel() != self.lib.mr_actor_param_count():
+            members = ddpg_population[0] if ddpg_population is not None else 1
+            if w.numel() != members * self.lib.mr_actor_param_count():
                 raise ValueError("actor tensor has the wrong number of parameters (use actor.pack_actor)")
             io.action_source = L.ACTIONS_ACTOR
             io.actor = w.data_ptr()
@@ -588,6 +593,8 @@ class VecMREnv:
             raise ValueError("give actions or policy")
         if ddpg_collect is not None and io.action_source != L.ACTIONS_ACTOR:
             raise ValueError("ddpg_collect needs an actor policy")
+        if ddpg_population is not None and ddpg_collect is None:
+            raise ValueError("ddpg_population needs ddpg_collect")
         io.k_steps = k
         res = {}
         if record_episodes:
@@ -623,13 +630,19 @@ class VecMREnv:
             res["done_traj"] = torch.empty(k, n, dtype=torch.uint8, device=self.device)
             io.traj_done = res["done_traj"].data_ptr()
         if accumulate_stats:
-            io.stats = self._stats.data_ptr()
+            io.stats = self._stats.data_ptr() if ddpg_population is None else ddpg_population[1].data_ptr()
         nz = self._noise_for(self.params.noise_var)
         if gp_pol is not None:
             rc = self.lib.mr_env_rollout_gp_heading(C.byref(self._c_state), n, self._dt, C.byref(self.params), C.byref(nz),
                                                     C.byref(self._c_tt), C.byref(io), C.byref(gp_pol), C.byref(self._c_out),
                                                     self._stream())
             L.check(rc, "mr_env_rollout_gp_heading")
+        elif ddpg_population is not None:
+            rc = self.lib.mr_env_rollout_ddpg_collect_population(C.byref(self._c_state), n, self._dt, C.byref(self.params),
+                                                                 C.byref(nz), C.byref(self._c_tt), C.byref(io),
+                                                                 C.byref(ddpg_collect), int(ddpg_population[0]),
+                                                                 C.byref(self._c_out), self._stream())
+            L.check(rc, "mr_env_rollout_ddpg_collect_population")
         elif ddpg_collect is not None:
             rc = self.lib.mr_env_rollout_ddpg_collect(C.byref(self._c_state), n, self._dt, C.byref(self.params), C.byref(nz),
                                                       C.byref(self._c_tt), C.byref(io), C.byref(ddpg_collect),
