@@ -556,6 +556,39 @@ int mr_env_rollout_ddpg_collect_population(const mr_env_state* st, int64_t n, in
                                            const mr_noise* nz, const mr_time_table* tt, const mr_rollout_io* io,
                                            const mr_ddpg_collect* c, int32_t members, const mr_step_out* out, void* stream);
 
+/* Greedy evaluation of a population: every member's actor, without exploration noise, on N fresh episodes, in ONE
+ * launch of the fused rollout over members x N envs.  Env i = p N + j plays episode j of member p:
+ *   - it starts from init[j] (or a sample of init_space, drawn as mr_env_reset draws it) with the reset of mr_env_reset
+ *     at step index nz->offset on an env whose previous model flag is p->is_mismatched, then steps K = max_timesteps + 1
+ *     times (step k at step index nz->offset + 1 + k) with a = mu(obs), exactly as mr_env_rollout with
+ *     MR_ACTIONS_ACTOR steps it;
+ *   - after its terminal step it takes no further steps and adds nothing; a tile whose envs have all ended stops.
+ * So member p's rows equal those of a solo env of N envs (auto_reset off; env_base nz->env_base with common random
+ * numbers, nz->env_base + p N without) that runs mr_env_reset(init) at step index nz->offset followed by mr_env_rollout
+ * with member p's actor and K steps, read at the first terminal step of each env: the same length and outcome, and the
+ * return bit for bit the sequential sum of that rollout's rewards (with float32 storage: of its unrounded rewards).
+ * Common random numbers (common_random_numbers = 1): env p N + j draws with the key of env j (Philox stream
+ * nz->env_base + j, column j of the noise table), so every member meets the same starts and noise.  Table noise: the
+ * table is [nz->table_len][table_cols] with table_cols >= N (common random numbers) or >= members N; every env's cursor
+ * starts at 0.  p->auto_reset is ignored; no state rows are read or written (there is no env state argument).  The
+ * actor path is that of mr_set_actor_path: 3xFP16 (default) or 3xTF32; the CUDA-core path returns MR_ERR_UNSUPPORTED.
+ * stats[p] receives, added: episodes N, the summed lengths and returns, the goal / out-of-bounds / timeout counts, the
+ * env steps taken and the envs with any status flag (MR_STAT_FAILED). */
+typedef struct mr_ddpg_eval {
+    const float* actors;            /* [members][mr_actor_param_count()]                                  */
+    int32_t members;                /* 1..MR_DDPG_MAX_MEMBERS                                             */
+    int32_t common_random_numbers;  /* 1: env p N + j draws what env j draws (keys, table column)         */
+    int64_t member_envs;            /* N, a positive multiple of 128                                      */
+    const void* init;               /* [N][2] storage dtype, or NULL: sample init_space                   */
+    double* stats;                  /* [members][MR_STATS_LEN], added to, or NULL                         */
+    double* ret; int32_t* length; uint8_t* outcome; uint8_t* status;   /* [members * N] each, or NULL    */
+    int64_t table_cols;             /* table noise: the row length of nz->table                           */
+} mr_ddpg_eval;
+/* outcome: 1 goal, 2 out of bounds, 3 timeout; status: the sticky MR_ENV_* flags of the episode (reset included).
+ * nz->offset_dev is not supported (MR_ERR_ARG). */
+int mr_ddpg_evaluate_population(const mr_ddpg_eval* ev, int32_t dtype, const mr_sim_params* p, const mr_noise* nz,
+                                const mr_time_table* tt, void* stream);
+
 /* mr_actor_forward for MR_Env observations — obs rows 2, 3 (the goal) are identically zero (MR_env.py:57) and are not
  * read — with the hidden layer on the tensor cores (tcgen05, 3xTF32 ~ fp32 accuracy).  Same arguments. */
 int mr_actor_forward_env(const float* actor, const void* obs, int64_t obs_row_stride, int64_t n, int32_t dtype,

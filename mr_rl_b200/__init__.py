@@ -9,6 +9,7 @@ Public surface (mirrors the reference's names):
     DDPGLearner, ReplayBuffer, OUNoise, ddpg.train   the DDPG learner of RL/MR_ddpg.py on the device
     ddpg.collect                  its acting loop (actor + OU noise + env step + replay add) fused into one rollout launch
     DDPGPopulation, PopulationReplay, ddpg.train_population   many independent learners, one update and one collect launch
+    evaluate_population, evaluate, pbt_plan, pbt_population   greedy evaluation of every member in one launch, and PBT on it
     init_actor / pack_actor / actor_forward   DDPG actor forward for the in-loop policy
     experiment_dict / save_experiment          recorded rollouts in the reference's MRExperiment pickle layout
 
@@ -17,7 +18,8 @@ there is no CPU fallback (importing is cheap, the first compute call loads the l
 """
 from ._lib import MRLibraryError, load as load_library  # noqa: F401
 from .actor import actor_forward, init_actor, pack_actor  # noqa: F401
-from .ddpg import DDPGLearner, DDPGPopulation, OUNoise, PopulationReplay, ReplayBuffer  # noqa: F401
+from .ddpg import (DDPGLearner, DDPGPopulation, OUNoise, PopulationEvaluation, PopulationReplay, ReplayBuffer, evaluate,  # noqa: F401
+                   evaluate_population, pbt_plan, pbt_population)
 from .gp import DeviceGP  # noqa: F401
 from .gpr import DeviceGPR  # noqa: F401
 from .learning_module import HeadingTrackingPolicy, LearningModule  # noqa: F401

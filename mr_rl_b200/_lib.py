@@ -112,6 +112,12 @@ class DDPGPopulation(C.Structure):
                 ("seeds", C.POINTER(C.c_uint64))]
 
 
+class DDPGEval(C.Structure):
+    _fields_ = [("actors", C.c_void_p), ("members", C.c_int32), ("common_random_numbers", C.c_int32),
+                ("member_envs", C.c_int64), ("init", C.c_void_p), ("stats", C.c_void_p), ("ret", C.c_void_p),
+                ("length", C.c_void_p), ("outcome", C.c_void_p), ("status", C.c_void_p), ("table_cols", C.c_int64)]
+
+
 GP_PAD = 128
 
 
@@ -122,7 +128,7 @@ EXPORTS = ("mr_abi_version", "mr_last_error", "mr_default_params", "mr_fill_time
            "mr_actor_forward", "mr_set_step_path", "mr_env_reset_ex", "mr_counter_set", "mr_set_actor_path",
            "mr_host_register", "mr_host_unregister", "mr_philox_normals", "mr_gp_correct_action_2d",
            "mr_env_rollout_gp_heading", "mr_env_rollout_ddpg_collect", "mr_ddpg_update_population",
-           "mr_env_rollout_ddpg_collect_population")
+           "mr_env_rollout_ddpg_collect_population", "mr_ddpg_evaluate_population")
 
 _lib = None
 
@@ -169,6 +175,8 @@ def load():
                                                            P(TimeTable), P(RolloutIO), P(DDPGCollect), C.c_int32, P(StepOut),
                                                            C.c_void_p]
     lib.mr_env_rollout_ddpg_collect_population.restype = C.c_int
+    lib.mr_ddpg_evaluate_population.argtypes = [P(DDPGEval), C.c_int32, P(SimParams), P(Noise), P(TimeTable), C.c_void_p]
+    lib.mr_ddpg_evaluate_population.restype = C.c_int
     lib.mr_ddpg_update_population.argtypes = [P(DDPGPopulation), C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p]
     lib.mr_ddpg_update_population.restype = C.c_int
     lib.mr_gp_predict.argtypes = [P(GPModel), C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,

@@ -265,9 +265,9 @@ static int do_rollout(const mr_env_state& st, int64_t n, const Params& p, const 
     const OutView<T> ov = out_view<T>(out, n);
     const NoiseView nv = noise_view(nz, n);
     switch (nz ? nz->mode : MR_NOISE_NONE) {
-        case MR_NOISE_TABLE: return launch_rollout<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, gh, cv, s);
-        case MR_NOISE_PHILOX: return launch_rollout<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, gh, cv, s);
-        default: return launch_rollout<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, gh, cv, s);
+        case MR_NOISE_TABLE: return launch_rollout<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, gh, cv, nullptr, s);
+        case MR_NOISE_PHILOX: return launch_rollout<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, gh, cv, nullptr, s);
+        default: return launch_rollout<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, gh, cv, nullptr, s);
     }
 }
 
@@ -685,4 +685,76 @@ extern "C" int mr_env_rollout_ddpg_collect_population(const mr_env_state* st, in
     cudaStream_t s = (cudaStream_t)stream;
     return dtype == MR_F64 ? mr::do_rollout<double>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s)
                            : mr::do_rollout<float>(*st, n, pp, nz, tv, *io, nullptr, &cv, out, s);
+}
+
+namespace mr {
+// the population evaluation through the fused rollout: no state rows, no outputs; the actors, the statistics rows, K and
+// the per-member env count N are all it takes besides the task
+template <class T>
+static int do_evaluate(const mr_ddpg_eval& e, const Params& p, const mr_noise* nz, const TimeView& tv, int k_steps,
+                       cudaStream_t s) {
+    StateView<T> sv;
+    memset(&sv, 0, sizeof(sv));
+    RolloutView<T> rv;
+    memset(&rv, 0, sizeof(rv));
+    rv.actor = e.actors; rv.stats = e.stats; rv.k_steps = k_steps; rv.action_source = MR_ACTIONS_ACTOR;
+    const int64_t n = (int64_t)e.members * e.member_envs;
+    const OutView<T> ov = out_view<T>(nullptr, n);
+    NoiseView nv = noise_view(nz, n);
+    nv.offset += 1;                                   // step k at offset + 1 + k; the kernel resets at offset
+    nv.table_stride = e.table_cols;
+    CollectView cv;
+    memset(&cv, 0, sizeof(cv));
+    cv.member_envs = e.member_envs;
+    EvalView<T> ev;
+    ev.init = (const T*)e.init; ev.ret = e.ret; ev.length = e.length; ev.outcome = e.outcome; ev.status = e.status;
+    ev.crn = e.common_random_numbers ? 1 : 0;
+    switch (nz->mode) {
+        case MR_NOISE_TABLE: return launch_rollout<T, MR_NOISE_TABLE>(sv, rv, ov, nv, tv, p, n, nullptr, &cv, &ev, s);
+        case MR_NOISE_PHILOX: return launch_rollout<T, MR_NOISE_PHILOX>(sv, rv, ov, nv, tv, p, n, nullptr, &cv, &ev, s);
+        default: return launch_rollout<T, MR_NOISE_NONE>(sv, rv, ov, nv, tv, p, n, nullptr, &cv, &ev, s);
+    }
+}
+}  // namespace mr
+
+extern "C" int mr_ddpg_evaluate_population(const mr_ddpg_eval* ev, int32_t dtype, const mr_sim_params* p, const mr_noise* nz,
+                                           const mr_time_table* tt, void* stream) {
+    mr::NvtxRange nvtx_range("mr_ddpg_evaluate_population");
+    using mr::fail;
+    const char* fn = "mr_ddpg_evaluate_population";
+    if (!ev || !p || !nz) return fail(MR_ERR_ARG, "%s: null evaluation, params or noise", fn);
+    if (!ev->actors) return fail(MR_ERR_ARG, "%s: null actor", fn);
+    if (ev->members < 1 || ev->members > MR_DDPG_MAX_MEMBERS)
+        return fail(MR_ERR_ARG, "%s: members must be in 1..%d", fn, MR_DDPG_MAX_MEMBERS);
+    // the tensor-core actor multiplies a whole 128-env tile by one weight matrix: a tile must not span two members
+    if (ev->member_envs <= 0 || ev->member_envs % 128 != 0 || ev->member_envs * ev->members > ((int64_t)1 << 31) - 1)
+        return fail(MR_ERR_ARG, "%s: member_envs must be a positive multiple of 128 (and members x member_envs < 2^31)", fn);
+    if (dtype != MR_F64 && dtype != MR_F32) return fail(MR_ERR_ARG, "%s: bad dtype %d", fn, dtype);
+    if (p->max_timesteps < 0) return fail(MR_ERR_ARG, "%s: max_timesteps must be >= 0", fn);
+    if (!(p->time_span > 0.0)) return fail(MR_ERR_ARG, "%s: time_span must be positive", fn);
+    const int k_steps = p->max_timesteps + 1;         // every episode ends within the launch
+    if (!tt || !tt->t || tt->len < 2 || tt->len < k_steps)
+        return fail(MR_ERR_ARG, "%s: the time table must hold at least max_timesteps + 1 = %d entries", fn, k_steps);
+    if (nz->offset_dev) return fail(MR_ERR_ARG, "%s: offset_dev is not supported (the step index is nz->offset)", fn);
+    const int mode = nz->mode;
+    if (mode != MR_NOISE_NONE && mode != MR_NOISE_TABLE && mode != MR_NOISE_PHILOX)
+        return fail(MR_ERR_ARG, "%s: unknown noise mode %d", fn, mode);
+    if (mode == MR_NOISE_NONE && p->noise_var != 0.0)
+        return fail(MR_ERR_ARG, "%s: noise_var=%g needs a noise source (table or philox)", fn, p->noise_var);
+    if (mode == MR_NOISE_TABLE) {
+        if (!nz->table || nz->table_len <= 0) return fail(MR_ERR_ARG, "%s: table noise without a table (table_len <= 0)", fn);
+        const int64_t cols = ev->common_random_numbers ? ev->member_envs : ev->member_envs * ev->members;
+        if (ev->table_cols < cols)
+            return fail(MR_ERR_ARG, "%s: the noise table has %lld columns, the evaluation reads %lld (%s)", fn,
+                        (long long)ev->table_cols, (long long)cols,
+                        ev->common_random_numbers ? "N with common random numbers" : "members x N");
+    }
+    if (mr::g_actor_path == 1)
+        return fail(MR_ERR_UNSUPPORTED, "%s: the CUDA-core actor path (mr_set_actor_path(1)) has no evaluation", fn);
+    mr::Params pp = mr::to_params(*p, nz);
+    pp.auto_reset = 0;
+    const mr::TimeView tv{tt->t, tt->len};
+    cudaStream_t s = (cudaStream_t)stream;
+    return dtype == MR_F64 ? mr::do_evaluate<double>(*ev, pp, nz, tv, k_steps, s)
+                           : mr::do_evaluate<float>(*ev, pp, nz, tv, k_steps, s);
 }

@@ -272,11 +272,23 @@ struct CollectView {
     int64_t capacity, head;         // transition (k, i) goes to slot (head + k n + i) % capacity
     int64_t member_envs;            // population (mr_env_rollout_ddpg_collect_population): envs per member N; 0: one learner
 };
+// Greedy evaluation of a DDPG population (mr_ddpg_evaluate_population): env i = p N + j (N = CollectView::member_envs)
+// starts episode j of member p in the launch and is frozen after its terminal step.  No state rows are read or written.
+template <class T>
+struct EvalView {
+    const T* init;              // [N][2] start positions, or NULL: sample init_space
+    double* ret;                // [n] undiscounted return, or NULL
+    int32_t* length;            // [n] episode length, or NULL
+    uint8_t* outcome;           // [n] 1 goal, 2 out of bounds, 3 timeout, or NULL
+    uint8_t* status;            // [n] sticky MR_ENV_* flags, or NULL
+    int crn;                    // common random numbers: env p N + j draws with the key of env j
+};
 // The fused rollout of every action source.  gh: the GP heading policy, only from mr_env_rollout_gp_heading; cv: the
-// DDPG collector, only from mr_env_rollout_ddpg_collect(_population); both null from mr_env_rollout.
+// DDPG collector, only from mr_env_rollout_ddpg_collect(_population); ev (with cv->member_envs): the population
+// evaluation, only from mr_ddpg_evaluate_population; all null from mr_env_rollout.
 template <class T, int MODE>
 int launch_rollout(const StateView<T>& sv, const RolloutView<T>& rv, const OutView<T>& ov, const NoiseView& nv,
                    const TimeView& tv, const Params& p, int64_t n, const GpHeadingView* gh, const CollectView* cv,
-                   cudaStream_t s);
+                   const EvalView<T>* ev, cudaStream_t s);
 
 }  // namespace mr

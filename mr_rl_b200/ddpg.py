@@ -5,12 +5,14 @@ Mirrors the reference's pieces with the same names and arguments where they exis
 ActorNetwork / CriticNetwork pair (:80-231) with their Adam optimisers and target networks, and ``train`` (:233-323)
 as a vectorised acting / learning loop.  One learner update (:285-305) is ONE kernel launch (csrc/mr_ddpg.cu).
 ``DDPGPopulation`` / ``PopulationReplay`` / ``train_population`` train many independent learners (seeds, sweeps) with one
-update launch and one collect launch for all of them.
+update launch and one collect launch for all of them; ``evaluate_population`` plays every member's greedy policy on fresh
+episodes in one launch, and ``pbt_population`` runs population-based training on top of it.
 Everything here fails without the CUDA library: there is no CPU path.
 """
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 import math
 
 import numpy as np
@@ -18,6 +20,7 @@ import torch
 
 from . import _lib as L
 from .actor import ORDER as ACTOR_ORDER, SHAPES as ACTOR_SHAPES, actor_forward, init_actor, pack_actor
+from .vec_env import raise_for_status
 
 CRITIC_ORDER = ("wc1", "bc1", "gc", "bec", "mc", "vc", "t1", "t1b", "t2", "t2b", "wo", "bo")
 CRITIC_SHAPES = {"wc1": (5, 64), "bc1": (64,), "gc": (64,), "bec": (64,), "mc": (64,), "vc": (64,),
@@ -377,6 +380,9 @@ def _per_member(name, v, members):
     return v
 
 
+_HYPER_FIELDS = (("actor_lr", "lr_actor"), ("critic_lr", "lr_critic"), ("tau", "tau"), ("gamma", "gamma"))
+
+
 def _check_members(members):
     members = int(members)
     if not 1 <= members <= L.DDPG_MAX_MEMBERS:
@@ -467,6 +473,48 @@ class DDPGPopulation:
         m.updates = self.updates
         return m
 
+    def hyper_table(self):
+        """The hyper-parameters as a [P, 4] float64 array, columns (actor_lr, critic_lr, tau, gamma)."""
+        return np.array([[getattr(h, f) for _, f in _HYPER_FIELDS] for h in self.hyper], dtype=np.float64)
+
+    def set_hyper(self, p, actor_lr=None, critic_lr=None, tau=None, gamma=None):
+        """Change member p's hyper-parameters (those given); its next update uses them.  ``member(p).hyper`` follows."""
+        p = self._index(p)
+        for (name, field), v in zip(_HYPER_FIELDS, (actor_lr, critic_lr, tau, gamma)):
+            if v is None:
+                continue
+            if not math.isfinite(float(v)):
+                raise ValueError(f"{name} must be finite")
+            setattr(self.hyper[p], field, float(v))
+            setattr(self._learners[p].hyper, field, float(v))
+
+    def exploit(self, dst, src):
+        """Member dst[k] becomes a copy of member src[k]: online and target actor and critic, the four Adam moments (one
+        index copy per stacked tensor, all sources read before any destination is written) and the hyper-parameters.
+        The destination keeps its sampling seed, replay ring, OU state and envs.  ``dst`` must not repeat a member."""
+        dst = [self._index(d) for d in np.atleast_1d(np.asarray(dst, dtype=np.int64))]
+        src = [self._index(s) for s in np.atleast_1d(np.asarray(src, dtype=np.int64))]
+        if len(dst) != len(src):
+            raise ValueError(f"dst has {len(dst)} members, src {len(src)}")
+        if len(set(dst)) != len(dst):
+            raise ValueError("dst repeats a member")
+        if not dst:
+            return
+        d = torch.tensor(dst, dtype=torch.int64, device=self.device)
+        s = torch.tensor(src, dtype=torch.int64, device=self.device)
+        for t in (self.actor, self.actor_target, self.critic, self.critic_target, *self._moments):
+            t.index_copy_(0, d, t.index_select(0, s))
+        rows = [L.DDPGHyper.from_buffer_copy(self.hyper[b]) for b in src]
+        for a, h in zip(dst, rows):
+            C.memmove(C.byref(self.hyper[a]), C.byref(h), C.sizeof(h))
+            C.memmove(C.byref(self._learners[a].hyper), C.byref(h), C.sizeof(h))
+
+    def _index(self, p):
+        p = int(p)
+        if not 0 <= p < self.members:
+            raise ValueError(f"member {p} is not in 0..{self.members - 1}")
+        return p
+
     def update(self, replay, batch_size=64):
         """One update of every member in ONE launch (one CTA per member): member p samples ``batch_size`` rows of its own
         ring, as DDPGLearner.update does with ``seed ^ random_seed``, and takes the single-CTA update (batch 1..4096).
@@ -525,12 +573,14 @@ def collect_population(env, pop, actor_noise, replay, k_steps, **rollout_kw):
 
 
 def train_population(env, pop, actor_noise, buffer_size=10000, min_batch=64, steps=1000, updates_per_step=1, replay=None,
-                     noise_var=1, a0=1, log_every=0, collect_steps=64):
+                     noise_var=1, a0=1, log_every=0, collect_steps=64, reset=True):
     """``train(collect_steps=K)`` for a population: per launch one ``collect_population`` of K env steps, then
     K * ``updates_per_step`` population updates once the rings hold ``min_batch`` transitions.  Returns the log
     [P, launches, 3]: per member the mean reward of the launch's transitions, and the loss and mean Q of its last update.
     With ``min_batch`` <= 64 member p's run equals its solo ``train(collect_steps=K)`` (above 64 samples the solo update
-    takes the data-parallel path, the population the single-CTA one)."""
+    takes the data-parallel path, the population the single-CTA one).  ``reset=False`` continues the env's episodes
+    instead of resetting it (``noise_var`` and ``a0`` are then unused): two calls of S and T steps, S a multiple of K, then
+    equal one call of S + T steps when they share ``replay``."""
     P = pop.members
     k = int(collect_steps)
     if k < 1:
@@ -541,7 +591,8 @@ def train_population(env, pop, actor_noise, buffer_size=10000, min_batch=64, ste
         raise ValueError(f"the replay has {replay.members} members, the population {P}")
     if N > replay.buffer_size:
         raise ValueError(f"{N} envs per member add more transitions per step than a member's replay buffer holds ({replay.buffer_size})")
-    env.reset(noise_var=noise_var, a0=a0)
+    if reset:
+        env.reset(noise_var=noise_var, a0=a0)
     launches = (steps + k - 1) // k
     log = torch.zeros(P, launches, 3, dtype=torch.float64, device=env.device)
     rew_sum = pop.stats[:, L.STAT_NAMES.index("sum_reward")]
@@ -561,3 +612,152 @@ def train_population(env, pop, actor_noise, buffer_size=10000, min_batch=64, ste
             print(f"launch {it + 1}/{launches} ({done} steps), mean over {P} members: reward {row[0]:.3f} "
                   f"critic loss {row[1]:.4g} mean Q {row[2]:.4g}")
     return log.cpu().numpy()
+
+
+# ---- greedy evaluation and population-based training ------------------------------------------------------------------
+
+@dataclasses.dataclass
+class PopulationEvaluation:
+    """What ``evaluate_population`` returns.  [P] device tensors, one value per member over its N episodes:
+    ``mean_return`` (undiscounted), ``goal_rate`` / ``out_of_bounds_rate`` / ``timeout_rate`` (how the episodes ended),
+    ``mean_length`` (steps), ``failed`` (episodes with a status flag) and ``env_steps`` (steps taken).  With ``per_env``
+    also the [P, N] rows ``ret`` (float64), ``length`` (int32), ``outcome`` (uint8: 1 goal, 2 out of bounds, 3 timeout)
+    and ``status`` (uint8, the sticky ENV_* flags); otherwise those are None."""
+    mean_return: torch.Tensor
+    goal_rate: torch.Tensor
+    out_of_bounds_rate: torch.Tensor
+    timeout_rate: torch.Tensor
+    mean_length: torch.Tensor
+    failed: torch.Tensor
+    env_steps: torch.Tensor
+    ret: torch.Tensor = None
+    length: torch.Tensor = None
+    outcome: torch.Tensor = None
+    status: torch.Tensor = None
+
+
+def evaluate_population(env, pop, member_envs, init=None, common_random_numbers=True, offset=0, per_env=False):
+    """Every member's greedy policy (its online actor, no exploration noise) on ``member_envs`` = N fresh episodes, in ONE
+    launch (mr_ddpg_evaluate_population).  ``env`` (any VecMREnv) supplies the task: storage dtype, noise kind, seed and
+    table, a0 / noise_var / is_mismatched, reward mode, bounds, max_timesteps and action bound; its state rows, statistics
+    and step index are not touched.  Episode j of every member starts at ``init[j]`` ([N, 2], or one (2,) position for
+    all), or at a sample of init_space, and runs to its end (at most max_timesteps + 1 steps).  ``offset`` is the Philox
+    step index of the evaluation: the start is drawn at ``offset`` and step k at ``offset + 1 + k``, as a solo env whose
+    step index is ``offset`` draws them on ``reset()`` followed by a rollout.  With ``common_random_numbers`` every
+    member's episode j draws what env j draws (so members differ only by their policies; a table then needs N columns),
+    without it env p N + j draws with key env_base + p N + j (a table needs P N columns).  Returns a PopulationEvaluation;
+    the stream is not synchronised.  ``mean_return`` is reduced from the per-env returns, so it does not depend on the
+    order of the launch's atomics."""
+    return _evaluate(env, pop.actor, pop.members, pop.action_bound, member_envs, init, common_random_numbers, offset, per_env)
+
+
+def evaluate(env, learner, n_envs, init=None, common_random_numbers=True, offset=0, per_env=False):
+    """``evaluate_population`` for one DDPGLearner on ``n_envs`` episodes (a multiple of 128); the result has P = 1."""
+    return _evaluate(env, learner.actor.reshape(1, -1), 1, learner.action_bound, n_envs, init, common_random_numbers, offset,
+                     per_env)
+
+
+def _evaluate(env, actors, members, action_bound, member_envs, init, crn, offset, per_env):
+    lib = L.load()
+    P = _check_members(members)
+    N = int(member_envs)
+    if N <= 0 or N % 128:
+        raise ValueError(f"member_envs = {N} must be a positive multiple of 128")
+    if tuple(action_bound) != (env.params.action_high[0], env.params.action_high[1]):
+        raise ValueError("the actors' action_bound must equal the env's action_space.high (the in-kernel actor scales by it)")
+    if env.per_env_params:
+        raise ValueError("the evaluation plays the env's launch parameters: envs with per-env parameter rows are not supported")
+    w = actors.to(device=env.device, dtype=torch.float32).contiguous()
+    if w.numel() != P * lib.mr_actor_param_count():
+        raise ValueError(f"the actors must be [{P}, {lib.mr_actor_param_count()}] (actor.pack_actor per member)")
+    init_t = None
+    if init is not None:
+        init_t = torch.as_tensor(np.asarray(init) if not torch.is_tensor(init) else init).to(device=env.device, dtype=env.dtype)
+        if init_t.dim() == 1 and init_t.numel() == 2:
+            init_t = init_t.reshape(1, 2).expand(N, 2)
+        init_t = init_t.contiguous()
+        if tuple(init_t.shape) != (N, 2):
+            raise ValueError(f"init must be (2,) or ({N}, 2)")
+    cols = 0
+    if env.noise_kind == "table":
+        cols = env._noise_table.shape[1]
+        need = N if crn else P * N
+        if cols < need:
+            raise ValueError(f"the noise table has {cols} columns; the evaluation reads {need} "
+                             f"({'N with' if crn else 'members x N without'} common random numbers)")
+    nz = L.Noise.from_buffer_copy(env._noise_for(env.params.noise_var))
+    nz.offset, nz.offset_dev = int(offset), None
+    dev = env.device
+    stats = torch.zeros(P, L.STATS_LEN, dtype=torch.float64, device=dev)
+    ret = torch.empty(P, N, dtype=torch.float64, device=dev)
+    rows = [torch.empty(P, N, dtype=dt, device=dev) for dt in (torch.int32, torch.uint8, torch.uint8)] if per_env else [None] * 3
+    ptr = lambda t: t.data_ptr() if t is not None else None
+    ev = L.DDPGEval(w.data_ptr(), P, 1 if crn else 0, N, ptr(init_t), stats.data_ptr(), ret.data_ptr(), *map(ptr, rows), cols)
+    with torch.cuda.device(dev):
+        rc = lib.mr_ddpg_evaluate_population(C.byref(ev), env._dt, C.byref(env.params), C.byref(nz), C.byref(env._c_tt),
+                                             _stream(dev))
+    L.check(rc, "mr_ddpg_evaluate_population")
+    col = lambda name: stats[:, L.STAT_NAMES.index(name)]
+    return PopulationEvaluation(mean_return=ret.mean(1), goal_rate=col("goal") / N, out_of_bounds_rate=col("out_of_bounds") / N,
+                                timeout_rate=col("timeout") / N, mean_length=col("sum_length") / N, failed=col("failed"),
+                                env_steps=col("env_steps"), ret=ret if per_env else None, length=rows[0], outcome=rows[1],
+                                status=rows[2])
+
+
+def pbt_plan(scores, fraction=0.25, perturb=(0.8, 1.25), rng=None):
+    """One exploit / explore decision of population-based training, on the host.  The members are ranked by ``scores``
+    (higher is better; equal scores rank by member index, lower first; NaN ranks last).  Each of the bottom
+    m = floor(fraction P) members copies a member drawn uniformly from the top m, and then multiplies its actor and critic
+    learning rates and tau by factors drawn from ``perturb``.  ``rng``: a numpy Generator or a seed.  Returns
+    (dst [m], src [m], factors [m, 3]) with dst in ranking order and factor columns (actor_lr, critic_lr, tau)."""
+    s = np.asarray(scores, dtype=np.float64).reshape(-1)
+    P = s.size
+    if not 0.0 <= float(fraction) <= 0.5:
+        raise ValueError("fraction must be in [0, 0.5] (the top and bottom fractions must not overlap)")
+    rng = np.random.default_rng(rng)
+    m = int(math.floor(float(fraction) * P))
+    order = np.lexsort((np.arange(P), -s))          # best first
+    dst = order[P - m:].astype(np.int64)
+    src = order[:m][rng.integers(0, m, size=m)].astype(np.int64) if m else np.zeros(0, dtype=np.int64)
+    factors = rng.choice(np.asarray(perturb, dtype=np.float64), size=(m, 3)) if m else np.zeros((0, 3))
+    return dst, src, factors
+
+
+def pbt_population(env, pop, actor_noise, replay, rounds, steps_per_round, eval_envs, fraction=0.25, perturb=(0.8, 1.25),
+                   seed=0, collect_steps=64, min_batch=64, eval_init=None):
+    """Population-based training.  Per round: ``train_population`` for ``steps_per_round`` steps (the first round resets
+    the env, later rounds continue its episodes and share ``replay``); ``evaluate_population`` with common random numbers
+    on ``eval_envs`` episodes per member (start positions ``eval_init`` or samples of init_space), at one Philox offset
+    per round drawn from ``seed``; then ``pbt_plan`` on the mean returns, ``pop.exploit(dst, src)`` and the perturbation of
+    the copied members' learning rates and tau.  Returns the history {"score": [R, P] mean returns, "hyper": [R, P, 4]
+    hyper-parameters the round trained with, "parent": [R, P] the member each member copied after the round (itself if
+    none)}.  Raises for the constant reward (every step earns 10, so the return ranks long episodes first) and when any
+    evaluation episode failed (as VecMREnv.check_status)."""
+    if env.params.reward_mode == L.REWARD_CONST10:
+        raise ValueError("population-based training ranks by return: the constant reward (10 per step) would favour "
+                         "policies that never reach the goal; use reward_mode='shaped'")
+    R, S = int(rounds), int(steps_per_round)
+    if R < 1 or S < 1:
+        raise ValueError("rounds and steps_per_round must be at least 1")
+    P = pop.members
+    if replay is None:
+        replay = PopulationReplay(P, 10000, 0, device=env.device)
+    rng = np.random.default_rng(seed)
+    score, hyper = np.zeros((R, P)), np.zeros((R, P, 4))
+    parent = np.tile(np.arange(P, dtype=np.int64), (R, 1))
+    for r in range(R):
+        train_population(env, pop, actor_noise, min_batch=min_batch, steps=S, replay=replay, collect_steps=collect_steps,
+                         reset=r == 0)
+        res = evaluate_population(env, pop, eval_envs, init=eval_init, common_random_numbers=True,
+                                  offset=int(rng.integers(0, 2**62)), per_env=True)
+        raise_for_status(res.status.reshape(-1))
+        score[r] = res.mean_return.cpu().numpy()
+        hyper[r] = pop.hyper_table()
+        dst, src, factors = pbt_plan(score[r], fraction, perturb, rng)
+        pop.exploit(dst, src)
+        table = pop.hyper_table()
+        for d, f in zip(dst, factors):
+            h = table[d]
+            pop.set_hyper(d, actor_lr=h[0] * f[0], critic_lr=h[1] * f[1], tau=h[2] * f[2])
+        parent[r, dst] = src
+    return {"score": score, "hyper": hyper, "parent": parent}

@@ -39,6 +39,19 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+def raise_for_status(status):
+    """Raise what the reference raises for the first failed envs of the sticky status flags ``status`` [N] (uint8)."""
+    flags = int(status.max().item()) if status.numel() else 0
+    if flags == 0:
+        return
+    idx = torch.nonzero(status)[:8, 0].tolist()
+    if flags & L.ENV_NOISE_OVERFLOW:
+        raise L.MRLibraryError(f"noise table exhausted for envs {idx}")
+    if flags & L.ENV_NONFINITE:
+        raise ValueError(f"non-finite state in envs {idx} (scipy: 'All components of the initial state `y0` must be finite')")
+    raise RuntimeError(f"integrator failed in envs {idx} (scipy: 'Attempt to step on a failed or finished solver')")
+
+
 class VecMREnv:
     """``num_envs`` independent MR_Env instances stepped by one kernel launch.
 
@@ -675,16 +688,7 @@ class VecMREnv:
 
     # ---- failure reporting: the reference raises from scipy; kernels set sticky flags ---------------
     def check_status(self):
-        bad = self._status[:self.num_envs]
-        flags = int(bad.max().item()) if self.num_envs else 0
-        if flags == 0:
-            return
-        idx = torch.nonzero(bad)[:8, 0].tolist()
-        if flags & L.ENV_NOISE_OVERFLOW:
-            raise L.MRLibraryError(f"noise table exhausted for envs {idx}")
-        if flags & L.ENV_NONFINITE:
-            raise ValueError(f"non-finite state in envs {idx} (scipy: 'All components of the initial state `y0` must be finite')")
-        raise RuntimeError(f"integrator failed in envs {idx} (scipy: 'Attempt to step on a failed or finished solver')")
+        raise_for_status(self._status[:self.num_envs])
 
     # ---- checkpoint / resume ----------------------------------------------------------------------------
     def state_dict(self):
